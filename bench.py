@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: my_model inference images/s (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One STEP = one pass of the four sub-networks' forward over one batch of synthetic inputs per
@@ -20,11 +20,20 @@ at 64 tiles per GPU, and `train.global_512` = global batch 512 as the config is 
 device next to their scipy.ndimage restatement on the host), `roofline`, `cpu_baseline`, `cpu_baseline_train`.
 Prints ONE JSON line (rank 0).
 
+`--steps K` is the number of timed steps of `value`, `e2e` (pipelined and synchronous), `train`,
+`train.global_512` and `fullpage`; `stages`, `tf32_long_gemm` and the per-layer `layers` breakdown repeat a fixed,
+small number of calls.
+
 No PyTorch: ranks rendezvous and reduce through libuocr's own NCCL binding (univer_ocr_b200.comm).
 
 `--impl reference` times the reference's CPU algorithm (oracle port: per-output-pixel NumPy
 loops, float64 -- what the reference's `_forward_cpu` / `_backward_cpu` do) on all host cores, one
 sample per core; see cpu_baseline.sample in its line.
+
+`--dump-outputs DIR` writes what the last timed step of `value` returned on rank 0 (the Paragraph, Line and Char
+predictions) as DIR/<name>.npy in float32, so that two builds can be compared output for output: inputs and weights
+are seeded, so the same arguments give the same inputs.  Above 64 MB in all, every array keeps the same fixed, seeded
+fraction of its leading-axis rows (tiles for Paragraph and Line, windows for Char), in order.
 """
 import argparse
 import ctypes
@@ -48,6 +57,7 @@ UNIT = 'images/s'
 # (nn/initializers.py:22-25) and saturates every output (sigmoid == 1.0: zero data gradient, constant loss); same
 # constants as the parity goldens (oracle/np_models.GOLDEN_SCALE)
 SIGNED_SCALE = {'monochrome': 5.0, 'paragraph': 5.5, 'line': 3.5, 'char': 2.5}
+DUMP_BYTES = 63 * 10**6               # array data of --dump-outputs; with the .npy headers the dump stays below 64 MB
 
 
 def load_peaks():
@@ -75,6 +85,19 @@ def synth_tiles(rng, n, hw):
 def synth_tiles_u8(rng, n, hw):
     """The same tiles as 8-bit image planes (what `encode_layers` divides by 255)."""
     return np.ascontiguousarray(np.rint(synth_tiles(rng, n, hw) * 255.0), dtype=np.uint8)
+
+
+def dump_outputs(directory, outputs, limit=DUMP_BYTES):
+    """Writes {name: float32 host array} as <directory>/<name>.npy.  Above `limit` bytes in all, every array keeps the
+    same fraction of its leading-axis rows, chosen by a fixed seed and kept in order."""
+    os.makedirs(directory, exist_ok=True)
+    total = sum(a.nbytes for a in outputs.values())
+    for name, a in outputs.items():
+        assert a.dtype == np.float32, (name, a.dtype)
+        if total > limit:
+            keep = max(1, a.shape[0] * limit // total)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(directory, name + '.npy'), a)
 
 
 def signed_init(model, scale, with_bias):
@@ -281,8 +304,17 @@ def run_b200(args):
         step(dev_sets[i % n_sets])
     sampler = ClockSampler(int(os.environ.get('LOCAL_RANK', '0')))
     sampler.start()
-    ms_per_step, launches = timer.device_ms(lambda i: step(dev_sets[i % n_sets]), args.steps)
+    last = []
+
+    def timed_step(i):
+        out = step(dev_sets[i % n_sets])
+        if i == args.steps - 1:
+            last.append(out)
+    ms_per_step, launches = timer.device_ms(timed_step, args.steps)
     value = B * comm.world / (ms_per_step / 1e3)
+    if args.dump_outputs and comm.rank == 0:
+        dump_outputs(args.dump_outputs, {name: o.get() for name, o in zip(('paragraph', 'line', 'char'), last[0])})
+    del last
 
     # ---------------- end to end through the public API with host buffers (`e2e`) ----------------
     # the pipelined public API (univer_ocr_b200.pipeline.InferencePipeline): H2D of batch i+1, forward of batch i and
@@ -334,7 +366,7 @@ def run_b200(args):
         e2e_sync(i)
     timer.barrier()
     sync_times = []
-    for i in range(max(5, args.steps // 2)):
+    for i in range(args.steps):
         t0 = time.perf_counter()
         e2e_sync(i)
         sync_times.append(time.perf_counter() - t0)
@@ -598,7 +630,7 @@ def measure_train(args, comm, timer, nn, my_model, models, dev_sets, rng, B):
                 'gpu_launches': launches, 'launch': launch_mode,
                 'losses_first_timed_step': first, 'losses_after': last}
 
-    steps = max(20, args.steps)
+    steps = args.steps
     feeds = {'monochrome': dev_sets[0]['page'], 'paragraph': dev_sets[0]['page'], 'line': dev_sets[0]['line'],
              'char': dev_sets[0]['char']}
     dps, step = build(B, models, feeds)
@@ -626,7 +658,9 @@ def measure_train(args, comm, timer, nn, my_model, models, dev_sets, rng, B):
             big = {'monochrome': pages, 'paragraph': pages, 'line': nn.CP.copy(synth_tiles(rng, per, LINE_HW)),
                    'char': nn.CP.copy(synth_tiles(rng, per, CHAR_HW))}
             dps, step = build(per, nets, big)
-            res = timed(step, max(5, min(steps, 2560 // per)), per, dps)
+            # K steps of batch 512 per GPU: at one GPU this section takes about K / 5 times as long as the five steps
+            # it once timed regardless of K
+            res = timed(step, steps, per, dps)
             res['scaling'] = 'strong'
             out['global_512'] = res
             del dps, step, nets, big, pages
@@ -718,11 +752,11 @@ def measure_fullpage(args, comm, timer, nn, my_model, rng):
             para.predict(mono.predict(sets[j % 2])[0])
     for _ in range(2):
         one_pass()
-    ms, launches = timer.device_ms(one_pass, 5)
+    ms, launches = timer.device_ms(one_pass, args.steps)
     done = launches_per_pass * per_launch * comm.world
     return {'metric': 'full-page inference pages/sec (2064x2064 after make_divisible_by, Monochrome->Paragraph)',
             'value': done / (ms / 1e3), 'unit': 'pages/s', 'pages_per_pass': done, 'pages_per_launch': per_launch,
-            'ms_per_pass': ms, 'passes_timed': 5, 'gpu_launches': launches, 'scaling': 'strong (64 pages over N GPUs)',
+            'ms_per_pass': ms, 'passes_timed': args.steps, 'gpu_launches': launches, 'scaling': 'strong (64 pages over N GPUs)',
             'l2_policy': 'two resident 4-page input sets (2 x 68 MB) alternate; 273 MB of intermediates per launch'}
 
 
@@ -855,7 +889,13 @@ def main():
     ap.add_argument('--no-fullpage', action='store_true', help='skip the full-page (configs[3]) measurement')
     ap.add_argument('--no-stages', action='store_true', help='skip the crop-stage (row f4) measurement')
     ap.add_argument('--no-gemm-peak', action='store_true', help='skip the long-GEMM TF32 rate measurement')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write the last timed step's predictions as DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the outputs of --impl b200')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     if args.impl == 'reference':
         run_reference(args)

@@ -1,12 +1,13 @@
 """TEST INFRASTRUCTURE ONLY -- loader for the *unmodified* reference (KerkDovan/univer-ocr).
 
-Imports the reference's `web_app.components.nn` (and `my_model.model`) straight from
-`/root/reference` under a handful of compatibility shims, so that its NumPy CPU path can be
-executed in the authoring container to (a) pin `oracle/np_oracle.py` and (b) generate the
-golden vectors committed under `tests/golden/`.
+Imports the reference's `web_app.components.nn` (and `my_model.model`) straight from the
+checkout that `UOCR_REFERENCE_ROOT` names, under a handful of compatibility shims, so that its
+NumPy CPU path can be executed to (a) pin `oracle/np_oracle.py` and (b) generate the golden
+vectors committed under `tests/golden/`.
 
-`/root/reference` does not exist on the GPU box: nothing that runs there may import this
-module (`available()` returns False there, and callers skip).
+The reference is not part of this repository: without `UOCR_REFERENCE_ROOT` pointing at a
+checkout of it, `available()` returns False and the live comparisons skip (the committed
+golden vectors keep checking what they recorded).
 
 Why shims are needed (reference targets Python 3.7 / NumPy 1.18 / CuPy 7):
   * `import cupy` at module top            -- nn/gpu.py:1, nn/gradient_check.py:3
@@ -14,7 +15,7 @@ Why shims are needed (reference targets Python 3.7 / NumPy 1.18 / CuPy 7):
   * `np.product`, `np.float`, `np.bool`    -- nn/layers/layers.py:298, nn/regularizations.py:6,
                                               nn/layers/maxpool.py:144
   * `web_app/__init__.py` imports Flask; `image_generator/generate.py:7` imports Faker
-Nothing under /root/reference is modified or copied.
+Nothing in the reference tree is modified or copied.
 """
 import collections
 import collections.abc
@@ -25,13 +26,13 @@ import types
 
 import numpy as np
 
-REFERENCE_ROOT = os.environ.get('UOCR_REFERENCE_ROOT', '/root/reference')
+REFERENCE_ROOT = os.environ.get('UOCR_REFERENCE_ROOT', '')
 
 _loaded = {}
 
 
 def available():
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, 'web_app', 'components', 'nn'))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, 'web_app', 'components', 'nn'))
 
 
 def _install_shims():
@@ -70,7 +71,7 @@ def load_nn():
     if 'nn' in _loaded:
         return _loaded['nn']
     if not available():
-        raise RuntimeError(f'reference tree not found at {REFERENCE_ROOT}')
+        raise RuntimeError(f'reference tree not found at {REFERENCE_ROOT!r}: set UOCR_REFERENCE_ROOT to a checkout of it')
     _install_shims()
     nn = importlib.import_module('web_app.components.nn')
     for sub in ('gpu', 'layers', 'losses', 'optimizers', 'regularizations', 'initializers',
@@ -97,7 +98,7 @@ def load_trainer():
     if 'trainer' in _loaded:
         return _loaded['trainer']
     if not available():
-        raise RuntimeError(f'reference tree not found at {REFERENCE_ROOT}')
+        raise RuntimeError(f'reference tree not found at {REFERENCE_ROOT!r}: set UOCR_REFERENCE_ROOT to a checkout of it')
     _install_shims()
     mod = importlib.import_module('web_app.components.my_model.trainer')
     _loaded['trainer'] = mod
@@ -116,7 +117,7 @@ def load_my_model_on(nn_package, alias='uocr_dropin'):
     if key in _loaded:
         return _loaded[key]
     if not available():
-        raise RuntimeError(f'reference tree not found at {REFERENCE_ROOT}')
+        raise RuntimeError(f'reference tree not found at {REFERENCE_ROOT!r}: set UOCR_REFERENCE_ROOT to a checkout of it')
     _install_shims()
     comp_dir = os.path.join(REFERENCE_ROOT, 'web_app', 'components')
     for pkg, path in ((alias, os.path.join(REFERENCE_ROOT, 'web_app')), (f'{alias}.components', comp_dir)):

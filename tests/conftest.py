@@ -13,7 +13,7 @@ GOLDEN_DIR = os.path.join(ROOT, 'tests', 'golden')
 
 def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA device (run on the B200 box)')
-    config.addinivalue_line('markers', 'reference: needs /root/reference (authoring container only)')
+    config.addinivalue_line('markers', 'reference: needs the reference tree named by UOCR_REFERENCE_ROOT')
 
 
 class Golden:

@@ -1,9 +1,9 @@
 """Generates tests/golden/glue.json by running the UNMODIFIED reference's PredToText._func1
 (interpreter/interpreter.py:595-614) and make_divisible_by (my_model/model.py:26-34) on seeded
 inputs.  The alphabet and the similar-character table are read from the reference's
-`primitives` package at generation time and stored as fixture data.  Authoring container only:
+`primitives` package at generation time and stored as fixture data.  Needs a checkout of the reference:
 
-    python tests/golden/make_glue_golden.py
+    UOCR_REFERENCE_ROOT=<reference checkout> python tests/golden/make_glue_golden.py
 """
 import importlib
 import json

@@ -1,7 +1,7 @@
 """Generates tests/golden/*.npz by executing the UNMODIFIED reference (NumPy CPU path) on seeded
-inputs.  Run in the authoring container only (needs /root/reference):
+inputs.  Needs a checkout of the reference:
 
-    python tests/golden/make_golden.py
+    UOCR_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden.py
 
 The reference has no stored vectors of its own (SURVEY.md 8c); its only fixed cases are the
 printed MaxPool / Upsample / Concat examples of nn/test/test_gradients.py:171-188,216-222,

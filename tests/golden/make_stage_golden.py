@@ -2,9 +2,9 @@
 (interpreter/interpreter.py: label_layer :16-22, rearrange_lines :41-84, rotate_array :188-192,
 FindObjectHeightInRotated._func :229-232, CropRotateAndZoomLines._func1 / _func2 :493-523, the ternary search of
 CropAndRotateSingleParagraph._func :318-343) on the seeded synthetic cases of tests/stage_cases.py.  Inputs are not
-stored: tests regenerate them from the same seeds.  Authoring container only:
+stored: tests regenerate them from the same seeds.  Needs a checkout of the reference:
 
-    python tests/golden/make_stage_golden.py
+    UOCR_REFERENCE_ROOT=<reference checkout> python tests/golden/make_stage_golden.py
 
 Boolean masks are cast to uint8 before the reference's own `ndimage.find_objects` calls (SciPy >= 1.18 refuses a boolean
 maximum label; the boxes are the same).  Arrays are handed over as float32, so the reference's float32 results are the

@@ -1,8 +1,8 @@
 """Generates tests/golden/trainer_traces.json by running the UNMODIFIED reference epoch driver
-(`my_model/trainer.py`) over the scripted scenarios of tests/trainer_cases.py.  Authoring
-container only (needs /root/reference):
+(`my_model/trainer.py`) over the scripted scenarios of tests/trainer_cases.py.  Needs a
+checkout of the reference:
 
-    python tests/golden/make_trainer_golden.py
+    UOCR_REFERENCE_ROOT=<reference checkout> python tests/golden/make_trainer_golden.py
 """
 import contextlib
 import io

@@ -4,8 +4,8 @@
 result is compared with what the repo's own mirror `univer_ocr_b200.my_model` builds: flattened layer names and
 order, relations, layer hyper-parameters, every intermediate output shape, parameter counts, fusion plans, the
 whole-network inference kernel and the fused-update eligibility.  Construction and shape analysis need no device
-(parameters are uploaded on first use), so this runs in the authoring container; it needs /root/reference and is
-skipped on the GPU box."""
+(parameters are uploaded on first use), so this runs without a GPU; it needs the reference tree (UOCR_REFERENCE_ROOT)
+and is skipped without it."""
 import os
 import sys
 
@@ -17,7 +17,7 @@ sys.path.insert(0, ROOT)
 
 from oracle import ref_loader  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason='needs /root/reference')
+pytestmark = pytest.mark.skipif(not ref_loader.available(), reason='needs the reference tree (UOCR_REFERENCE_ROOT)')
 
 SHAPES = {'monochrome': (2, 496, 736, 1), 'paragraph': (2, 496, 736, 1), 'line': (2, 128, 256, 1),
           'char': (2, 32, 256, 1)}

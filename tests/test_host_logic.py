@@ -180,7 +180,7 @@ def test_receptive_field_matches_reference_values():
     assert rf['Paragraph/down_1/conv_1']['input 0']['cnt'] == (5, 5)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason='/root/reference not present')
+@pytest.mark.skipif(not ref_loader.available(), reason='needs the reference tree (UOCR_REFERENCE_ROOT)')
 def test_flattening_matches_reference_model():
     """Same nested construction through the reference's own Model: identical leaf names,
     relations and receptive fields."""
@@ -192,6 +192,22 @@ def test_flattening_matches_reference_model():
     mine._order = mine._resolve_order()
     mine.is_initialized = True
     assert ref.get_receptive_fields() == mine.get_receptive_fields()
+
+
+@pytest.mark.parametrize('name', ['monochrome', 'paragraph', 'line', 'char'])
+def test_builders_match_reference_parameters_golden(golden, name):
+    """What the reference's own builders produced, as tests/golden/models.npz recorded it (make_golden.py builds each
+    network with the reference's make_*): every parameter's flattened name, in the reference's order, and the
+    network's output shape.  my_model's builders must give the same, with no device."""
+    import univer_ocr_b200.nn as nn
+    from tests.cases import MODEL_SHAPES
+    from univer_ocr_b200 import my_model
+    g = golden('models').case(name)
+    want = [k[len('grad1__'):-len('__val')] for k in g if k.startswith('grad1__') and k.endswith('__val')]
+    shape = MODEL_SHAPES[name]
+    model = my_model.MAKERS[name](shape, optimizer=nn.optimizers.Adam(lr=0.0015))
+    assert [k.replace('/', '.') for k in model.params()] == want and len(want) >= 4
+    assert tuple(model.get_output_shapes([shape])[0]) == g['pred0'].shape
 
 
 def test_multi_output_submodel_tuple_sources():

@@ -2,8 +2,8 @@
 
 1. Against the committed golden vectors (tests/golden/*.npz, produced by running the
    unmodified reference -- see tests/golden/make_golden.py).  Runs everywhere.
-2. Live, against the reference imported from /root/reference, on fresh random inputs
-   (`-m reference`-style tests; auto-skipped where the tree is absent, e.g. the GPU box).
+2. Live, against the reference imported from the tree UOCR_REFERENCE_ROOT names, on fresh
+   random inputs (`-m reference`-style tests; skipped where that tree is absent).
 
 Tolerance: both sides are float64, only summation order differs -> rtol 1e-10.
 """
@@ -202,13 +202,15 @@ def test_thresholded_is_mean_max_midpoint_per_image_and_channel():
 
 # ------------------------------------------------------------------ live reference diffs
 
-needs_ref = pytest.mark.skipif(not ref_loader.available(), reason='/root/reference not present')
+needs_ref = pytest.mark.skipif(not ref_loader.available(), reason='needs the reference tree (UOCR_REFERENCE_ROOT)')
 
 
 @needs_ref
 @pytest.mark.reference
 @pytest.mark.parametrize('seed', [1, 2])
 def test_live_conv_pool_against_reference(seed):
+    """Fresh random inputs through the reference's layers.  Without the reference tree, test_conv_golden and
+    test_maxpool_golden check the same oracle functions against what the reference computed."""
     nn = ref_loader.load_nn()
     rng = np.random.default_rng(seed)
     for ks, pad, pv, st in (((3, 3), 1, 0.5, 1), ((5, 5), 2, 0.0, 2), ((5, 3), (0, 1), 0.0, (2, 1)),
@@ -280,7 +282,10 @@ def test_stage_oracle_matches_reference_functions():
     """The stage restatements of oracle/np_stages.py against the reference's own functions (interpreter.py:
     label_layer, rearrange_lines, CropRotateAndZoomLines._func1 / _func2, FindObjectHeightInRotated._func,
     rotate_array) on the synthetic cases of tests/stage_cases.py, all four reading directions.  Boolean masks are cast
-    to uint8 before the reference's find_objects calls (SciPy 1.18 refuses a boolean maximum label)."""
+    to uint8 before the reference's find_objects calls (SciPy 1.18 refuses a boolean maximum label).  Without the
+    reference tree, test_stage_oracle_matches_reference_golden checks the line counts, the line crops (zoomed to height 32,
+    minimal width 200; they depend on rearrange_lines and line_region), the paragraph angles (the end of the ternary
+    search) and the paragraph crops against tests/golden/stages.npz."""
     import importlib
     from scipy import ndimage
     from oracle import np_stages as S

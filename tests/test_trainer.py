@@ -1,6 +1,6 @@
 """Epoch driver (SURVEY.md 8f row 1): `univer_ocr_b200.trainer.Trainer` against traces of the
 reference's `my_model/trainer.py` on scripted models (tests/golden/trainer_traces.json, generated
-by tests/golden/make_trainer_golden.py; compared live as well where /root/reference exists), plus
+by tests/golden/make_trainer_golden.py; compared live as well where UOCR_REFERENCE_ROOT names the reference tree), plus
 the batched / sharded behaviour the reference does not have."""
 import contextlib
 import io
@@ -37,6 +37,8 @@ def test_golden_traces_cover_the_rollback_branches():
 
 
 def test_trainer_matches_reference_live():
+    """The golden traces against the reference itself.  Without the reference tree, test_trainer_matches_reference_trace
+    checks the same scenarios against tests/golden/trainer_traces.json."""
     from oracle import ref_loader
     if not ref_loader.available():
         pytest.skip('reference tree not present')

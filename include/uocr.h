@@ -190,9 +190,10 @@ int uocr_weights_to_kmajor(const float* w, float* wt, int64_t k_rows, int64_t n_
  * (inference only: nothing is saved for a backward pass).   replaces: the conv_1 -> leaky_relu_1
  * -> conv_2 -> sigmoid chain of make_monochrome (my_model/model.py:119-122), i.e. four
  * layer calls of convolutional.py:62-99 / layers.py:390-415.   x, y: (N, H, W, 1).
- * math_mode TF32 with c_mid == 16 runs BOTH convolutions on the tensor cores (tcgen05.mma with the A operands
- * resident in tensor memory, csrc/conv_pair_tc.cu); UOCR_PAIR_TC=0 in the environment keeps the CUDA-core
- * kernel, UOCR_PAIR_TC=1 selects the earlier shared-memory MMA variant (a measured negative result). */
+ * math_mode TF32 with c_mid == 16 runs BOTH convolutions on the tensor cores (tcgen05.mma): a persistent kernel
+ * whose first convolution reads the image rows in shared memory directly (csrc/conv_pair_rows_tc.cu; W % 4 == 0,
+ * W >= 8, 16-byte aligned x), otherwise the kernel that keeps its A operands in tensor memory (csrc/conv_pair_tc.cu).
+ * math_mode FP32 and c_mid != 16 run the CUDA-core kernel. */
 int uocr_conv3x3_pair_fwd(const float* x, const float* w1, const float* b1, const float* w2,
                           const float* b2, float* y, int64_t n, int64_t h, int64_t w, int32_t c_mid,
                           int act1, float alpha1, int act2, float alpha2, int math_mode, void* stream);
@@ -208,9 +209,8 @@ int uocr_conv3x3_pair_fwd(const float* x, const float* w1, const float* b1, cons
  * its input shape); UOCR_ERR_UNSUPPORTED otherwise.  FP32 FFMA in every math mode. */
 int uocr_hourglass1_fwd(const float* x, const float* const* weights, const float* const* biases, float* y,
                         int64_t n, int64_t h, int64_t w, float alpha, int act_end, float alpha_end, void* stream);
-/* the same with a math mode: UOCR_MATH_TF32 runs the network's full-resolution levels as tcgen05.mma straight from the
- * intermediate maps in shared memory (TF32 operands, FP32 accumulators in tensor memory; tolerance 1e-3 of the output
- * range); UOCR_MATH_FP32 is uocr_hourglass1_fwd. */
+/* the same with a math mode, for callers that carry one: both modes run the same FP32 FFMA kernel, so the result is
+ * bit-identical to uocr_hourglass1_fwd. */
 int uocr_hourglass1_fwd_mode(const float* x, const float* const* weights, const float* const* biases, float* y,
                              int64_t n, int64_t h, int64_t w, float alpha, int act_end, float alpha_end,
                              int math_mode, void* stream);

@@ -629,16 +629,23 @@ def test_inference_pipeline_matches_direct_predict(nn, graph):
         got[tag] = outs[0].copy()
     assert sorted(got) == list(range(7))
     for i in range(7):
-        assert np.array_equal(got[i], want[i]), i@pytest.mark.gpu
+        assert np.array_equal(got[i], want[i]), i
+
+
+@pytest.mark.gpu
 def test_hourglass_fused_kernel_vs_oracle(nn):
     """uocr_hourglass1_fwd (the whole Paragraph network in one kernel, parity-folded upsample convs)
     vs the float64 oracle chain of five conv layers, for block-aligned, ragged (H, W not multiples of
-    the 32 x 128 block), tiny and full-tile sizes; FP32 tolerance (rtol 1e-4 + 2e-6 max)."""
+    the 32 x 128 block), tiny and full-tile sizes, and one grid large enough for the 64-row blocks
+    (5 x 512 x 2048: 640 blocks of 64 x 128); FP32 tolerance (rtol 1e-4 + 2e-6 max).
+    uocr_hourglass1_fwd_mode runs the same kernel in both math modes: TF32 mode is bit-identical."""
     import ctypes
-    from univer_ocr_b200._lib import ACT_NONE, ACT_SIGMOID, lib
+    from univer_ocr_b200._lib import ACT_NONE, ACT_SIGMOID, MATH_TF32, lib
     rng = np.random.default_rng(123)
     for (n, h, w), act_end in (((2, 32, 128), ACT_SIGMOID), ((1, 36, 140), ACT_NONE), ((3, 4, 4), ACT_SIGMOID),
-                               ((2, 8, 300), ACT_NONE), ((1, 132, 12), ACT_SIGMOID), ((1, 496, 736), ACT_SIGMOID)):
+                               ((2, 8, 300), ACT_NONE), ((1, 132, 12), ACT_SIGMOID), ((1, 496, 736), ACT_SIGMOID),
+                               ((2, 496, 736), ACT_SIGMOID), ((1, 64, 2064), ACT_SIGMOID),
+                               ((5, 512, 2048), ACT_SIGMOID)):
         X = f32(rng.uniform(size=(n, h, w, 1)))
         ws = [f32(rng.standard_normal((5, 5, 1, 1)) * 0.25) for _ in range(5)]
         bs = [f32(rng.standard_normal(1) * 0.3) for _ in range(5)]
@@ -657,6 +664,10 @@ def test_hourglass_fused_kernel_vs_oracle(nn):
         lib.uocr_hourglass1_fwd(dX.ptr, ptrs(*[a.ptr for a in dw]), ptrs(*[a.ptr for a in db]), y.ptr, n, h, w,
                                 0.01, act_end, 0.0, nn.CP.stream())
         close(host(y), want, 1e-4, 2e-6, f'hourglass {(n, h, w)}')
+        y_tf32 = nn.DeviceArray.full((n, h, w, 1), -3.0)
+        lib.uocr_hourglass1_fwd_mode(dX.ptr, ptrs(*[a.ptr for a in dw]), ptrs(*[a.ptr for a in db]), y_tf32.ptr, n, h,
+                                     w, 0.01, act_end, 0.0, MATH_TF32, nn.CP.stream())
+        assert np.array_equal(host(y_tf32), host(y)), f'hourglass tf32 mode {(n, h, w)}'
 
 
 @pytest.mark.gpu

@@ -84,12 +84,13 @@ def test_fc_tf32_rounding_is_unbiased(nn):
 
 @pytest.mark.parametrize('shape,cin,cout,ks,pad,st', [
     ((3, 14, 256), 64, 64, (5, 3), (0, 1), (2, 1)),      # Char conv_2
+    ((64, 14, 256), 64, 64, (5, 3), (0, 1), (2, 1)),     # Char conv_2 at full batch
     ((3, 5, 256), 64, 64, (5, 3), (0, 1), (2, 1)),       # Char conv_3
     ((2, 14, 70), 64, 64, (5, 3), (0, 1), (2, 1)),       # ragged width (partial 128-pixel tile)
     ((2, 9, 131), 32, 48, (3, 3), (1, 1), (1, 1)),       # other channel counts / square kernel
     ((2, 11, 67), 32, 64, (3, 3), (1, 1), (1, 1)),       # Cin 32: four taps per wgrad CTA
     ((1, 9, 40), 128, 32, (2, 3), (1, 1), (2, 1)),       # Cin 128: one tap per wgrad CTA, even kernel height
-], ids=['char2', 'char3', 'ragged', 'c32_48', 'c32_64', 'c128_32'])
+], ids=['char2', 'char2_b64', 'char3', 'ragged', 'c32_48', 'c32_64', 'c128_32'])
 def test_conv_tf32(nn, shape, cin, cout, ks, pad, st):
     rng = np.random.default_rng(sum(shape) + cin)
     n, h, w = shape
@@ -106,21 +107,6 @@ def test_conv_tf32(nn, shape, cin, cout, ks, pad, st):
     close_tf32(dX, odX, 'dX')
     close_tf32(layer.w.grad, odW, 'dW')
     close_tf32(layer.b.grad, odb, 'db')
-
-
-def test_conv_slab_multicast_cluster_variant(nn, monkeypatch):
-    """UOCR_CONV_SLAB_MC=1: the two x-blocks of a 256-pixel output row as a thread-block cluster that shares the weight
-    chunks by TMA multicast (csrc/tc_gemm.cu: tc_conv_slab_kernel<true>; slower than the plain kernel, off by default, kept
-    as a measured negative result) -- same results as the oracle at Char conv_2 / conv_3 geometry."""
-    monkeypatch.setenv('UOCR_CONV_SLAB_MC', '1')
-    rng = np.random.default_rng(99)
-    for (n, h, w) in ((64, 14, 256), (3, 5, 256)):
-        X = f32(rng.standard_normal((n, h, w, 64)))
-        wt = f32(rng.standard_normal((5, 3, 64, 64)) / np.sqrt(15 * 64))
-        b = f32(rng.standard_normal(64))
-        layer = nn.layers.Convolutional2D((5, 3), 64, 64, padding=(0, 1), stride=(2, 1), w=wt, b=b)
-        y = layer.forward(X)[0]
-        close_tf32(y, O.conv2d_fwd(X, wt, b, (0, 1), 0.0, (2, 1)), f'multicast slab {(n, h, w)}')
 
 
 def test_char_model_tf32_matches_fp32(nn):
@@ -145,10 +131,10 @@ def test_char_model_tf32_matches_fp32(nn):
 def test_monochrome_pair_on_tensor_cores(nn):
     """uocr_conv3x3_pair_fwd in TF32 mode vs the float64 oracle: |err| <= 1e-3 * max (outputs are sigmoid values in
     (0, 1)) for aligned and ragged sizes (tile / strip / band / step remainders, single-pixel rows and columns,
-    odd image counts, several work units per persistent CTA), plus agreement with the FP32 pair kernel.  Variants:
-    `rows` (default, csrc/conv_pair_rows_tc.cu: GEMM 1 reads the image rows in shared memory through overlapping
-    descriptor rows; needs W % 4 == 0, otherwise the next variant runs), `tmem` (csrc/conv_pair_tc.cu: windows
-    stored to tensor memory), `smem` (the earlier shared-memory MMA variant, a measured negative result)."""
+    odd image counts, several work units per persistent CTA), plus agreement with the FP32 pair kernel.  TF32 mode
+    runs csrc/conv_pair_rows_tc.cu (GEMM 1 reads the image rows in shared memory through overlapping descriptor rows)
+    where W % 4 == 0 and W >= 8; the other widths (150, 3, 1, 31, 61, 734) take csrc/conv_pair_tc.cu (windows stored to
+    tensor memory), 9 x 300 x 734 at several bands per image."""
     import ctypes
     from univer_ocr_b200._lib import ACT_LEAKY, ACT_NONE, ACT_SIGMOID, lib
     rng = np.random.default_rng(17)
@@ -156,7 +142,8 @@ def test_monochrome_pair_on_tensor_cores(nn):
                             ((2, 1, 1), ACT_NONE), ((1, 63, 31), ACT_SIGMOID), ((1, 130, 61), ACT_NONE),
                             ((5, 3, 240), ACT_SIGMOID), ((2, 496, 736), ACT_SIGMOID), ((3, 33, 244), ACT_SIGMOID),
                             ((2, 40, 248), ACT_NONE), ((1, 7, 492), ACT_SIGMOID), ((1, 130, 1000), ACT_SIGMOID),
-                            ((5, 3, 12), ACT_NONE), ((1, 2, 8), ACT_SIGMOID), ((9, 300, 736), ACT_SIGMOID)):
+                            ((5, 3, 12), ACT_NONE), ((1, 2, 8), ACT_SIGMOID), ((9, 300, 736), ACT_SIGMOID),
+                            ((9, 300, 734), ACT_NONE)):
         X = f32(rng.uniform(size=(n, h, w, 1)))
         w1 = f32(rng.standard_normal((3, 3, 1, 16)) * 0.4)
         b1 = f32(rng.standard_normal(16) * 0.2)
@@ -168,14 +155,10 @@ def test_monochrome_pair_on_tensor_cores(nn):
             want = O.sigmoid_fwd(want)
         d = [nn.CP.copy(a) for a in (X, w1, b1, w2, b2)]
         outs = {}
-        # math mode 0 = FP32 pair kernel; mode 1 with UOCR_PAIR_TC = 2 (default): both convs as tcgen05.mma with
-        # TMEM-resident operands; = 1: the earlier shared-memory MMA variant (kept as a measured negative result)
-        for key, mode, variant, grid in (('fp32', 0, None, None), ('rows', 1, '3', None), ('rows_1cta', 1, '3', '1'),
-                                         ('rows_5cta', 1, '3', '5'), ('tmem', 1, '2', None), ('smem', 1, '1', None)):
-            if key.startswith('rows_') and n * h * w > 2000000:
+        # math mode 0 = FP32 pair kernel, 1 = tensor cores; the capped grids put many work units on each CTA
+        for key, mode, grid in (('fp32', 0, None), ('tf32', 1, None), ('tf32_1cta', 1, '1'), ('tf32_5cta', 1, '5')):
+            if grid is not None and n * h * w > 2000000:
                 continue                                # the capped-grid runs exist for the multi-unit bookkeeping
-            if variant is not None:
-                os.environ['UOCR_PAIR_TC'] = variant
             if grid is not None:
                 os.environ['UOCR_PAIR_ROWS_GRID'] = grid      # few persistent CTAs: many work units per CTA
             try:
@@ -184,7 +167,6 @@ def test_monochrome_pair_on_tensor_cores(nn):
                                           ACT_LEAKY, 0.01, act2, 0.0, mode, nn.CP.stream())
                 outs[key] = np.asarray(y.get(), dtype=np.float64)
             finally:
-                os.environ.pop('UOCR_PAIR_TC', None)
                 os.environ.pop('UOCR_PAIR_ROWS_GRID', None)
         for key in outs:
             if key == 'fp32':
@@ -387,44 +369,6 @@ def test_monochrome_pair_backward_tensor_core(nn):
                 for name, a, b in zip(('dw1', 'db1', 'dw2', 'db2', 'dx'), outs[1], (odw1, odb1, odw2, odb2, odx)):
                     close_tf32(a, np.asarray(b, dtype=np.float64).reshape(a.shape),
                                f'pair bwd tc vs oracle {name} {(n, h, w)} exact={exact}', tol=tol)
-
-
-def test_hourglass_tensor_core_levels_vs_oracle(nn, monkeypatch):
-    """uocr_hourglass1_fwd_mode in TF32 mode with UOCR_HOURGLASS_TC=1: the Paragraph network's `end` level as
-    tcgen05.mma straight from the U1 block in shared memory (csrc/hourglass.cu; slower than the FFMA level, kept as a
-    measured negative result and therefore off by default) -- vs the float64 oracle chain of five conv layers and vs
-    the FP32 kernel, for block-aligned, ragged, tiny and full-tile sizes.  Tolerance 1e-3 of the output range (2e-3 for
-    the un-squashed linear output, whose range is the sum of five layers' gains)."""
-    monkeypatch.setenv('UOCR_HOURGLASS_TC', '1')
-    import ctypes
-    from univer_ocr_b200._lib import ACT_NONE, ACT_SIGMOID, lib
-    rng = np.random.default_rng(321)
-    for (n, h, w), act_end in (((2, 32, 128), ACT_SIGMOID), ((1, 36, 140), ACT_NONE), ((3, 4, 4), ACT_SIGMOID),
-                               ((2, 8, 300), ACT_NONE), ((1, 132, 12), ACT_SIGMOID), ((2, 496, 736), ACT_SIGMOID),
-                               ((1, 64, 2064), ACT_SIGMOID)):
-        X = f32(rng.uniform(size=(n, h, w, 1)))
-        ws = [f32(rng.standard_normal((5, 5, 1, 1)) * 0.25) for _ in range(5)]
-        bs = [f32(rng.standard_normal(1) * 0.3) for _ in range(5)]
-        t = O.leaky_relu_fwd(O.conv2d_fwd(X, ws[0], bs[0], 2, stride=2), 0.01)
-        t = O.leaky_relu_fwd(O.conv2d_fwd(t, ws[1], bs[1], 2, stride=2), 0.01)
-        t = O.leaky_relu_fwd(O.conv2d_fwd(O.upsample2d_fwd(t, 2), ws[2], bs[2], 2), 0.01)
-        t = O.leaky_relu_fwd(O.conv2d_fwd(O.upsample2d_fwd(t, 2), ws[3], bs[3], 2), 0.01)
-        want = O.conv2d_fwd(t, ws[4], bs[4], 2)
-        if act_end == ACT_SIGMOID:
-            want = O.sigmoid_fwd(want)
-        dX = nn.CP.copy(X)
-        dw = [nn.CP.copy(a) for a in ws]
-        db = [nn.CP.copy(a) for a in bs]
-        ptrs = ctypes.c_void_p * 5
-        outs = {}
-        for mode in (0, 1):
-            y = nn.DeviceArray.full((n, h, w, 1), -3.0)
-            lib.uocr_hourglass1_fwd_mode(dX.ptr, ptrs(*[a.ptr for a in dw]), ptrs(*[a.ptr for a in db]), y.ptr, n, h, w,
-                                         0.01, act_end, 0.0, mode, nn.CP.stream())
-            outs[mode] = np.asarray(y.get(), dtype=np.float64)
-        tol = 1e-3 if act_end == ACT_SIGMOID else 2e-3
-        close_tf32(outs[1], want, f'hourglass tf32 vs oracle {(n, h, w)}', tol=tol)
-        close_tf32(outs[1], outs[0], f'hourglass tf32 vs fp32 {(n, h, w)}', tol=tol)
 
 
 def _line_oracle(X, ws, bs, act_end, alpha=0.01, alpha_end=0.0):

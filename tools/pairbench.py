@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Monochrome conv pair: TF32 tensor-core kernel vs the FP32 CUDA-core kernel (correctness + time).
-    UOCR_PAIR_TC=2 UOCR_PAIR_OCC=7 UOCR_PAIR_RB=30 python tools/pairbench.py [--batch 64]
+    python tools/pairbench.py [--batch 64] [--iters 10] [--h 496] [--w 736]
 """
 import argparse
 import ctypes
@@ -64,9 +64,7 @@ def main():
         px = n * h * w
         med = float(np.median(ts))
         print(f'mode {"tf32" if mode else "fp32"}: median {med:.4f} ms  best {min(ts):.4f} ms  '
-              f'{8 * px / med / 1e6:.0f} GB/s  {2 * 288 * px / med / 1e9:.1f} TFLOP/s '
-              f'(env TC={os.environ.get("UOCR_PAIR_TC")} OCC={os.environ.get("UOCR_PAIR_OCC")} '
-              f'RB={os.environ.get("UOCR_PAIR_RB")})', flush=True)
+              f'{8 * px / med / 1e6:.0f} GB/s  {2 * 288 * px / med / 1e9:.1f} TFLOP/s', flush=True)
     err = np.abs(outs[1] - outs[0])
     print(f'max |tf32 - fp32| = {err.max():.3e} (mean {err.mean():.3e}, signed mean {(outs[1] - outs[0]).mean():.3e})')
     bad = np.argwhere(err > 2e-3)

@@ -1,7 +1,8 @@
 #!/usr/bin/env python
-"""Monochrome conv pair, row-GEMM kernel (UOCR_PAIR_TC=3, csrc/conv_pair_rows_tc.cu): correctness against the FP32
-CUDA-core kernel over ragged shapes, then time at batch 64 next to the TMEM-window kernel (UOCR_PAIR_TC=2).
-    python tools/pairrows_check.py [--quick]
+"""Monochrome conv pair in TF32 mode (the row-GEMM kernel, csrc/conv_pair_rows_tc.cu, where W % 4 == 0; the
+TMEM-window kernel, csrc/conv_pair_tc.cu, otherwise): correctness against the FP32 CUDA-core kernel over ragged shapes,
+then the time of the TF32 dispatch at batch 64.
+    python tools/pairrows_check.py [--quick] [--multi] [--notime]
 """
 import ctypes
 import os
@@ -54,7 +55,6 @@ for g, (n, h, w) in [(g_, sh) for g_ in grids for sh in shapes]:
     for act1, act2 in ((ACT_LEAKY, ACT_SIGMOID), (ACT_LEAKY, ACT_NONE), (ACT_NONE, ACT_SIGMOID)):
         ref = nn.DeviceArray((n, h, w, 1))
         run(d, ref, n, h, w, 0, act1, act2)
-        os.environ['UOCR_PAIR_TC'] = '3'
         got = nn.DeviceArray.full((n, h, w, 1), -7.0)
         run(d, got, n, h, w, 1, act1, act2)
         a, b = got.get().astype(np.float64), ref.get().astype(np.float64)
@@ -72,22 +72,20 @@ if '--notime' in sys.argv:
 n, h, w = 64, 496, 736
 d = problem(n, h, w)
 flush = nn.DeviceArray((64 * 1024 * 1024,))
-for tc in ('2', '3'):
-    os.environ['UOCR_PAIR_TC'] = tc
-    y = nn.DeviceArray((n, h, w, 1))
-    for _ in range(3):
-        run(d, y, n, h, w, 1)
-    ts = []
-    for _ in range(10):
-        flush.fill(0)
-        e0, e1 = event(), event()
-        lib.uocr_event_record(e0, stream)
-        run(d, y, n, h, w, 1)
-        lib.uocr_event_record(e1, stream)
-        lib.uocr_event_sync(e1)
-        ms = ctypes.c_float(0)
-        lib.uocr_event_elapsed_ms(e0, e1, ctypes.byref(ms))
-        ts.append(ms.value)
-    t = float(np.median(ts))
-    print(f'UOCR_PAIR_TC={tc}: {t * 1e3:.1f} us per 64 tiles  ({186.9e6 / t / 1e6:.0f} GB/s algorithmic, '
-          f'{186.9e6 / t / 1e6 / 6547.8 * 100:.1f} % of HBM peak)', flush=True)
+y = nn.DeviceArray((n, h, w, 1))
+for _ in range(3):
+    run(d, y, n, h, w, 1)
+ts = []
+for _ in range(10):
+    flush.fill(0)
+    e0, e1 = event(), event()
+    lib.uocr_event_record(e0, stream)
+    run(d, y, n, h, w, 1)
+    lib.uocr_event_record(e1, stream)
+    lib.uocr_event_sync(e1)
+    ms = ctypes.c_float(0)
+    lib.uocr_event_elapsed_ms(e0, e1, ctypes.byref(ms))
+    ts.append(ms.value)
+t = float(np.median(ts))
+print(f'tf32 pair: {t * 1e3:.1f} us per 64 tiles  ({186.9e6 / t / 1e6:.0f} GB/s algorithmic, '
+      f'{186.9e6 / t / 1e6 / 6547.8 * 100:.1f} % of HBM peak)', flush=True)

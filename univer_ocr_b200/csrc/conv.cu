@@ -395,22 +395,14 @@ int uocr_conv3x3_pair_fwd(const float* x, const float* w1, const float* b1, cons
     UOCR_REQUIRE(h < (1 << 30) && w < (1 << 30), "dimension too large");
     UOCR_REQUIRE(act1 >= UOCR_ACT_NONE && act1 <= UOCR_ACT_SIGMOID && act2 >= UOCR_ACT_NONE &&
                      act2 <= UOCR_ACT_SIGMOID, "unknown activation");
-    // TF32 mode, c_mid == 16: tensor-core variants.  UOCR_PAIR_TC = 3 (default): GEMM 1 reads the image rows in
-    // shared memory through overlapping descriptor rows, persistent warp-specialised kernel (conv_pair_rows_tc.cu;
-    // needs w % 4 == 0, else variant 2 runs); 2: both convolutions as tcgen05.mma with windows stored to tensor
-    // memory (conv_pair_tc.cu); 1: the earlier variant whose hidden tile is evaluated on the CUDA cores and only the
-    // 16 -> 1 convolution runs as MMA from shared memory (kept as a measured negative result, 3x slower than the
-    // CUDA-core kernel); 0: CUDA-core pair kernel.
-    const char* pair_env = getenv("UOCR_PAIR_TC");       // read per call: tests switch between the variants
-    const int pair_tc = pair_env ? atoi(pair_env) : 3;
-    if (math_mode == UOCR_MATH_TF32 && pair_tc) {
-        int rc = UOCR_ERR_UNSUPPORTED;
-        if (pair_tc == 3)      // GEMM 1 straight from the image rows in shared memory (conv_pair_rows_tc.cu)
-            rc = conv3x3_pair_rows(x, w1, b1, w2, b2, y, n, h, w, c_mid, act1, alpha1, act2, alpha2, as_stream(stream));
+    // TF32 mode, c_mid == 16: on the tensor cores.  First the persistent warp-specialised kernel whose GEMM 1 reads the
+    // image rows in shared memory through overlapping descriptor rows (conv_pair_rows_tc.cu); where that one has no
+    // kernel (w % 4 != 0, w < 8, unaligned x, ...), the one that stores both convolutions' windows to tensor memory
+    // (conv_pair_tc.cu).  FP32 mode and every other shape: the CUDA-core pair kernel.
+    if (math_mode == UOCR_MATH_TF32) {
+        int rc = conv3x3_pair_rows(x, w1, b1, w2, b2, y, n, h, w, c_mid, act1, alpha1, act2, alpha2, as_stream(stream));
         if (rc == UOCR_ERR_UNSUPPORTED)
-            rc = pair_tc >= 2
-                ? conv3x3_pair_tmem(x, w1, b1, w2, b2, y, n, h, w, c_mid, act1, alpha1, act2, alpha2, as_stream(stream))
-                : conv3x3_pair_tc(x, w1, b1, w2, b2, y, n, h, w, c_mid, act1, alpha1, act2, alpha2, as_stream(stream));
+            rc = conv3x3_pair_tmem(x, w1, b1, w2, b2, y, n, h, w, c_mid, act1, alpha1, act2, alpha2, as_stream(stream));
         if (rc != UOCR_ERR_UNSUPPORTED) return rc;
     }
     return conv3x3_pair_fwd(x, w1, b1, w2, b2, y, n, h, w, c_mid, act1, alpha1, act2, alpha2,

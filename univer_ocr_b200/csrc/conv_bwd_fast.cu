@@ -696,8 +696,7 @@ int conv_wgrad_fast(const ConvGeom& g, int math_mode, const float* x, const floa
         const int rc = conv_wgrad_tc(g, x, dy, dw, db, accumulate, st);
         if (rc != UOCR_ERR_UNSUPPORTED) return rc;
     }
-    static const bool tiled = [] { const char* e = getenv("UOCR_WGRAD_TILED"); return !e || e[0] != '0'; }();
-    if (tiled && ws && wgrad_tiled_ok(g) && !((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dy)) & 15)) {
+    if (ws && wgrad_tiled_ok(g) && !((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dy)) & 15)) {
         const int64_t ntiles = (int64_t)g.n * ceil_div(g.ho, WT_TY) * ceil_div(g.wo, WT_TX);
         const int nblk = (int)(ntiles < wgrad_tiled_grid() ? ntiles : wgrad_tiled_grid());
         const size_t smem = sizeof(float) * ((WT_TY + 4) * (WT_TX + 4) * 4 + WT_TY * WT_TX * g.cout);
@@ -770,8 +769,8 @@ int conv_wgrad_fast(const ConvGeom& g, int math_mode, const float* x, const floa
 // ------------------------------------------------------------------------------------------
 constexpr int PB_CW = 8, PB_R = 16, PB_THREADS = 128;
 
-template <int CW, int R, int MINB>
-__global__ void __launch_bounds__(PB_THREADS, MINB) conv3x3_pair_wgrad_kernel(
+template <int CW, int R>
+__global__ void __launch_bounds__(PB_THREADS, 4) conv3x3_pair_wgrad_kernel(
     const float* __restrict__ x, const float* __restrict__ w1, const float* __restrict__ b1,
     const float* __restrict__ w2, const float* __restrict__ dy, float* __restrict__ ws, int n_img, int H, int W,
     int C1, int act1, float alpha1, int nblk) {
@@ -1016,27 +1015,17 @@ int conv3x3_pair_bwd(const float* x, const float* w1, const float* b1, const flo
     const int64_t nblk = ceil_div(items, PB_THREADS);
     if (nblk > 0x7fffffff) return UOCR_ERR_UNSUPPORTED;
     const size_t smem = sizeof(float) * 20 * c1;
-    static const bool wgrad_tc = [] { const char* e = getenv("UOCR_PAIR_WGRAD_TC"); return !e || e[0] != '0'; }();
-    int tc_nblk = 0;
-    if (math_mode == UOCR_MATH_TF32 && wgrad_tc &&
-        conv3x3_pair_wgrad_tc(x, w1, b1, w2, dy, ws, n, h, w, c1, act1, alpha1, &tc_nblk, st) == UOCR_OK) {
-        // tensor-core assisted weight gradients (conv_pair_bwd_tc.cu); same workspace layout, same finalize
-        conv3x3_pair_wgrad_finalize_kernel<<<(c1 + 1) * 19, 256, 0, st>>>(ws, tc_nblk, c1, dw1, db1, dw2, db2, accumulate);
-        UOCR_LAUNCHED("conv3x3_pair_wgrad_finalize");
-        if (dx) {
-            conv3x3_pair_dgrad_kernel<PB_CW, PB_R><<<(unsigned)nblk, PB_THREADS, smem, st>>>(
-                x, w1, b1, w2, dy, dx, (int)n, (int)h, (int)w, c1, act1, alpha1);
-            UOCR_LAUNCHED("conv3x3_pair_dgrad");
-        }
-        return UOCR_OK;
+    // TF32 mode: tensor-core assisted weight gradients (conv_pair_bwd_tc.cu) where they have a kernel; same workspace
+    // layout, same finalize
+    int wgrad_nblk = 0;
+    if (!(math_mode == UOCR_MATH_TF32 &&
+          conv3x3_pair_wgrad_tc(x, w1, b1, w2, dy, ws, n, h, w, c1, act1, alpha1, &wgrad_nblk, st) == UOCR_OK)) {
+        conv3x3_pair_wgrad_kernel<PB_CW, PB_R><<<(unsigned)nblk, PB_THREADS, smem, st>>>(
+            x, w1, b1, w2, dy, ws, (int)n, (int)h, (int)w, c1, act1, alpha1, (int)nblk);
+        UOCR_LAUNCHED("conv3x3_pair_wgrad");
+        wgrad_nblk = (int)nblk;
     }
-    static const int minb = [] { const char* e = getenv("UOCR_PAIRBWD_MINB"); return e ? atoi(e) : 4; }();
-#define PB_LAUNCH(MB) conv3x3_pair_wgrad_kernel<PB_CW, PB_R, MB><<<(unsigned)nblk, PB_THREADS, smem, st>>>( \
-        x, w1, b1, w2, dy, ws, (int)n, (int)h, (int)w, c1, act1, alpha1, (int)nblk)
-    if (minb >= 5) PB_LAUNCH(5); else if (minb == 4) PB_LAUNCH(4); else PB_LAUNCH(3);
-#undef PB_LAUNCH
-    UOCR_LAUNCHED("conv3x3_pair_wgrad");
-    conv3x3_pair_wgrad_finalize_kernel<<<(c1 + 1) * 19, 256, 0, st>>>(ws, (int)nblk, c1, dw1, db1, dw2, db2, accumulate);
+    conv3x3_pair_wgrad_finalize_kernel<<<(c1 + 1) * 19, 256, 0, st>>>(ws, wgrad_nblk, c1, dw1, db1, dw2, db2, accumulate);
     UOCR_LAUNCHED("conv3x3_pair_wgrad_finalize");
     if (dx) {
         conv3x3_pair_dgrad_kernel<PB_CW, PB_R><<<(unsigned)nblk, PB_THREADS, smem, st>>>(

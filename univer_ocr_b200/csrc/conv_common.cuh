@@ -32,9 +32,6 @@ int conv_wgrad_fast(const ConvGeom& g, int math_mode, const float* x, const floa
 int conv_fwd_tc(const ConvGeom& g, const float* x, const float* w, const float* w_kmajor /* (Cout, K) or NULL */,
                 const float* b, float* y, int act, float alpha, cudaStream_t st);
 
-int conv3x3_pair_tc(const float* x, const float* w1, const float* b1, const float* w2, const float* b2, float* y,
-                    int64_t n, int64_t h, int64_t w, int c1, int act1, float alpha1, int act2, float alpha2,
-                    cudaStream_t st);
 // 5x5 / stride 1 / Cin = 4 forward as a row GEMM on tcgen05 with TMEM-resident windows (conv_row_tc.cu)
 int conv55_row_tc(const ConvGeom& g, const float* x, const float* w, const float* b, float* y, int act, float alpha,
                   cudaStream_t st);

@@ -543,8 +543,7 @@ int conv_fwd_fast(const ConvGeom& g, int ups, int math_mode, const float* x, con
         int rc = conv_fwd_tc(g, x, w, w_kmajor, b, y, act, alpha, st);
         if (rc != UOCR_ERR_UNSUPPORTED) return rc;
         // 5x5 / stride 1 / Cin = 4 (Line up_*, end): row GEMM with TMEM-resident windows (conv_row_tc.cu)
-        static const bool row_tc = [] { const char* e = getenv("UOCR_ROW_TC"); return !e || e[0] != '0'; }();
-        if (row_tc && g.ups == ups) {
+        if (g.ups == ups) {
             rc = conv55_row_tc(g, x, w, b, y, act, alpha, st);
             if (rc != UOCR_ERR_UNSUPPORTED) return rc;
         }

@@ -354,11 +354,6 @@ __global__ void __launch_bounds__(PM_THREADS, 4) conv3x3_pair_tmem_kernel(const 
     }
 }
 
-static int env_int_pm(const char* name, int dflt) {
-    const char* e = getenv(name);
-    return e ? atoi(e) : dflt;
-}
-
 int conv3x3_pair_tmem(const float* x, const float* w1, const float* b1, const float* w2, const float* b2, float* y,
                       int64_t n, int64_t h, int64_t w, int c1, int act1, float alpha1, int act2, float alpha2,
                       cudaStream_t st) {
@@ -368,16 +363,12 @@ int conv3x3_pair_tmem(const float* x, const float* w1, const float* b1, const fl
     // output rows per band: a multiple of PM_R minus the 2 halo rows keeps every step full
     // (measured on 64 tiles of 496 x 736: 126-row bands 0.133 ms, 62 rows 0.139, 30 rows 0.155; shorter bands only
     // when there would otherwise be fewer than ~2 waves of CTAs, 4 resident per SM)
-    static const int rb_env = env_int_pm("UOCR_PAIR_RB", 0);
     PairTcParams p{};
     p.x = x; p.w1 = w1; p.b1 = b1; p.w2 = w2; p.b2 = b2; p.y = y;
     p.H = (int)h; p.W = (int)w;
     p.strips = (int)ceil_div(w, PM_OUT);
-    int rb = rb_env;
-    if (rb <= 0) {
-        rb = 126;
-        while (rb > 14 && n * ceil_div(h, rb) * p.strips / 4 < 2 * 4 * 148) rb = rb / 2 - 1;    // 126, 62, 30, 14
-    }
+    int rb = 126;
+    while (rb > 14 && n * ceil_div(h, rb) * p.strips / 4 < 2 * 4 * 148) rb = rb / 2 - 1;    // 126, 62, 30, 14
     p.rb = (int)(h < rb ? h : rb);
     p.bands = (int)ceil_div(h, p.rb);
     p.items = n * p.bands * p.strips;

@@ -232,17 +232,13 @@ int conv55_row_tc(const ConvGeom& g, const float* x, const float* w, const float
     if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15) return UOCR_ERR_UNSUPPORTED;
     // output rows per band: tall bands amortise the 4 halo rows, short ones give enough CTAs for a few waves
     // (4 resident per SM); measured on the Line shapes: 12 rows beat 28 and 60 there
-    static const int rb_env = [] { const char* e = getenv("UOCR_ROWTC_RB"); return e ? atoi(e) : 0; }();
     RowTcParams p{};
     p.x = x; p.w = w; p.b = g.bias ? b : nullptr; p.y = y;          // no bias: the stride-1 dgrad on flipped weights
     p.H = g.h; p.W = g.w;
     p.strips = (int)ceil_div(g.w, 32);
-    int rb = rb_env;
-    if (rb <= 0) {
-        rb = 12;
-        for (int cand : {60, 28}) {
-            if ((int64_t)g.n * ceil_div(g.h, cand) * p.strips / 4 >= 3 * 4 * 148) { rb = cand; break; }
-        }
+    int rb = 12;
+    for (int cand : {60, 28}) {
+        if ((int64_t)g.n * ceil_div(g.h, cand) * p.strips / 4 >= 3 * 4 * 148) { rb = cand; break; }
     }
     p.rb = g.h < rb ? g.h : rb;
     p.bands = (int)ceil_div(g.h, p.rb);

@@ -41,43 +41,21 @@ constexpr int HG_WSLOT = 28;
 
 template <int TH, int TW>
 struct HG {
-    // X block: origin column ox0 - 16 (16-byte aligned for cp.async; the convolution reads from column 2 on),
-    // two spare rows for the last 4-row strip of D1
+    // X block: origin column ox0 - 16 (16-byte aligned rows; the convolution reads from column 2 on), two spare rows
+    // for the last 4-row strip of D1
     static constexpr int XH = TH + 25, XW = TW + 27, XP = (XW + 1 + 3) & ~3, XROWS = XH + 2;
     static constexpr int D1H = TH / 2 + 11, D1W = TW / 2 + 11, D1P = (D1W + 3 + 3) & ~3;
     static constexpr int D2H = TH / 4 + 4, D2W = TW / 4 + 4, D2P = (D2W + 2 + 3 + 3) & ~3;
     static constexpr int U2H = TH / 2 + 4, U2W = TW / 2 + 4, U2P = (U2W + 3 + 3) & ~3;
     static constexpr int U1H = TH + 4, U1W = TW + 4, U1P = (U1W + 3 + 3) & ~3;
-    static constexpr int FLOATS = XROWS * XP + D1H * D1P + D2H * D2P + U2H * U2P + U1H * U1P + 5 * HG_WSLOT + 2 * 36 + 6;
-    // FFMA kernel: the U1 block lives in the x block, which is dead after down_1 -- 54.6 KB, 4 CTAs / SM
-    static constexpr int FLOATS_ALIASED = FLOATS - U1H * U1P;
+    // the U1 block lives in the x block, which is dead after down_1 -- 54.6 KB, 4 CTAs / SM
+    static constexpr int FLOATS = XROWS * XP + D1H * D1P + D2H * D2P + U2H * U2P + 5 * HG_WSLOT + 2 * 36 + 6;
     static_assert(U1H * U1P <= XROWS * XP, "U1 fits into the x block");
-    // tensor-core `end` level (TF32 mode): the U1 block is read as a tcgen05 A operand whose row m is the 8 floats
-    // from float 4 m of the block on (rows of the descriptor overlap; `position` m = row m / PPR, columns 4 (m % PPR) ..
-    // + 3).  M tiles of 128 positions cover the TH output rows; the last tile's rows run past the block (garbage lanes):
-    // END_PAD floats of slack keep those reads inside the CTA's allocation.
-    static constexpr int PPR = U1P / 4;                                  // positions per block row
-    static constexpr int END_TILES = (TH * PPR + 127) / 128;
-    static constexpr int END_B = 5 * 2 * 16 * 4;                         // B operand: 5 kernel rows x 2 chunks x 16 x 4
-    // floats past the end of the U1 block that the last tile's (garbage) rows read: the weights, folded kernels and
-    // barrier behind the block absorb 5 * HG_WSLOT + 2 * 36 + 6 of them, END_PAD floats of slack the rest.  The B operand
-    // lives in the X block, which is dead after down_1: 3 CTAs / SM need <= ~2 KB of extra shared memory per CTA
-    // (with the B operand appended the kernel dropped to 2 CTAs / SM and ran 1.5x slower, measured).
-    static constexpr int END_OVER = END_TILES * 128 * 4 + 4 * U1P + 8 - U1H * U1P;
-    static constexpr int END_PAD = END_OVER > 5 * HG_WSLOT + 78 ? ((END_OVER - (5 * HG_WSLOT + 78) + 3) & ~3) : 0;
-    static constexpr int FLOATS_TC = ((FLOATS + 3) & ~3) + END_PAD + 8;
-    static_assert(END_B <= XROWS * XP, "the B operand of the tensor-core level reuses the X block");
 };
 
 constexpr int HG_THREADS = 256;
 // 64-row blocks run with 512 threads (2 CTAs / SM = the same 32 warps): 7 % fewer halo FMAs, half the prologues
 __host__ __device__ constexpr int hg_threads(int th) { return th >= 64 ? 512 : HG_THREADS; }
-
-__device__ __forceinline__ bool elect_one_hg() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0;
-}
 
 template <int N4>
 __device__ __forceinline__ void hg_load_weights(const float* __restrict__ src, float* w) {
@@ -179,7 +157,7 @@ __device__ __forceinline__ void hg_down_pairs(const float* __restrict__ src, flo
 // dst (DH x DW at 2x the source resolution, origin (gy0, gx0) even) = act(conv5x5(upsample2(src)) + b) through the four
 // parity-folded 3 x 3 kernels wf[py][px][a][b]; output rows (2j, 2j+1) x columns (2n, 2n+1) read src(j + a, n + b).
 // Thread = 2 source cells = a 2 x 4 output block (8-byte loads, 16-byte stores at lane stride: conflict-free).
-template <int DH, int DW, int DP, int SP, int NT, bool ROUND_TF32 = false>
+template <int DH, int DW, int DP, int SP, int NT>
 __device__ __forceinline__ void hg_up(const float* __restrict__ src, float* __restrict__ dst, const float* __restrict__ wf,
                                       float bias, int gy0, int gx0, int hl, int wl, float alpha) {
     float w[36];
@@ -207,7 +185,6 @@ __device__ __forceinline__ void hg_up(const float* __restrict__ src, float* __re
 #pragma unroll
                         for (int b = 0; b < 3; ++b) acc = fmaf(w[((py * 2 + px) * 3 + a) * 3 + b], s[a][i + b], acc);
                     o[2 * i + px] = fmaxf(acc, acc * alpha);
-                    if (ROUND_TF32) o[2 * i + px] = round_tf32(o[2 * i + px]);     // the map is a tcgen05 A operand next
                 }
             const bool rowin = (unsigned)(gy0 + 2 * j + py) < (unsigned)hl;
 #pragma unroll
@@ -233,8 +210,8 @@ __device__ __forceinline__ void hg_fold(const float* __restrict__ w25, float* __
     }
 }
 
-template <int TH, int TW, bool TMA, bool TC>
-__global__ void __launch_bounds__(hg_threads(TH), TH >= 64 ? 2 : (TC ? 3 : 4)) hourglass1_fwd_kernel(const HourglassParams p,
+template <int TH, int TW>
+__global__ void __launch_bounds__(hg_threads(TH), TH >= 64 ? 2 : 4) hourglass1_fwd_kernel(const HourglassParams p,
                                                                        const __grid_constant__ CUtensorMap map_x) {
     using G = HG<TH, TW>;
     constexpr int NT = hg_threads(TH);
@@ -243,42 +220,23 @@ __global__ void __launch_bounds__(hg_threads(TH), TH >= 64 ? 2 : (TC ? 3 : 4)) h
     float* sD1 = sX + G::XROWS * G::XP;
     float* sD2 = sD1 + G::D1H * G::D1P;
     float* sU2 = sD2 + G::D2H * G::D2P;
-    float* sU1 = TC ? sU2 + G::U2H * G::U2P : sX;    // FFMA kernel: over the x block (dead after down_1)
-    float* sW = sU2 + G::U2H * G::U2P + (TC ? G::U1H * G::U1P : 0);     // 5 x (25 weights + bias)
+    float* sU1 = sX;                                 // over the x block (dead after down_1)
+    float* sW = sU2 + G::U2H * G::U2P;               // 5 x (25 weights + bias)
     float* sF = sW + 5 * HG_WSLOT;                   // folded kernels of up_2, up_1
 
     const int ox0 = blockIdx.x * TW, oy0 = blockIdx.y * TH;
-    const float* xim = p.x + (int64_t)blockIdx.z * p.H * p.W;
     float* yim = p.y + (int64_t)blockIdx.z * p.H * p.W;
     const int tid = threadIdx.x;
 
-    // ---- level 0: x block -> shared memory.  TMA: ONE thread issues one 3-D box (XP x XH x 1 at (ox0 - 16, oy0 - 14,
-    // image)); out-of-image elements arrive as zeros (= the padding), completion on an mbarrier.  The cp.async variant
-    // (zero fill through src-size 0) spent 18 % of the kernel's instructions on addresses and bounds (ncu source view).
+    // ---- level 0: x block -> shared memory.  ONE thread issues one 3-D TMA box (XP x XH x 1 at (ox0 - 16, oy0 - 14,
+    // image)); out-of-image elements arrive as zeros (= the padding), completion on an mbarrier.  A per-thread cp.async
+    // fill (zero fill through src-size 0) spent 18 % of the kernel's instructions on addresses and bounds (ncu source view).
     uint64_t* bar = reinterpret_cast<uint64_t*>(sF + 2 * 36);          // 8-byte aligned: all segment sizes are even
-    if (TMA) {
-        if (tid == 0) {
-            mbar_init(smem_u32(bar), 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            mbar_arrive_expect_tx(smem_u32(bar), (uint32_t)(G::XH * G::XP * sizeof(float)));
-            tma_load_3d(smem_u32(sX), &map_x, smem_u32(bar), ox0 - 16, oy0 - 14, (int)blockIdx.z);
-        }
-    } else {
-        constexpr int QUADS = G::XP / 4;
-        const uint32_t sbase = static_cast<uint32_t>(__cvta_generic_to_shared(sX));
-        // (r, q) advance by HG_THREADS quads per iteration without a division
-        constexpr int DR = NT / QUADS, DQ = NT % QUADS;
-        int r = tid / QUADS, q = tid - r * QUADS;
-        for (; r < G::XH; ) {
-            const int gy = oy0 - 14 + r, gx = ox0 - 16 + 4 * q;
-            const bool in = (unsigned)gy < (unsigned)p.H && (unsigned)gx < (unsigned)p.W;
-            const float* gsrc = in ? xim + (int64_t)gy * p.W + gx : xim;
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;"
-                         ::"r"(sbase + (uint32_t)(r * G::XP + 4 * q) * 4u), "l"(gsrc), "r"(in ? 16 : 0) : "memory");
-            r += DR; q += DQ;
-            if (q >= QUADS) { q -= QUADS; ++r; }
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
+    if (tid == 0) {
+        mbar_init(smem_u32(bar), 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_arrive_expect_tx(smem_u32(bar), (uint32_t)(G::XH * G::XP * sizeof(float)));
+        tma_load_3d(smem_u32(sX), &map_x, smem_u32(bar), ox0 - 16, oy0 - 14, (int)blockIdx.z);
     }
     // weights: static level index (a runtime index into p.w[] forces the whole parameter block into local memory)
     if (tid < 26) {
@@ -287,102 +245,18 @@ __global__ void __launch_bounds__(hg_threads(TH), TH >= 64 ? 2 : (TC ? 3 : 4)) h
     }
     // the two spare rows the last strip of D1 reads must be finite
     for (int i = tid; i < 2 * G::XP; i += NT) sX[G::XH * G::XP + i] = 0.f;
-    float* sBend = sX;                                                   // TC only: written once the X block is dead
-    uint64_t* bar_mma = reinterpret_cast<uint64_t*>(hg_smem + ((G::FLOATS + 3) & ~3) + G::END_PAD);
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar_mma + 2);
-    if (TC) {
-        if (tid == 0) {                                  // one barrier per round of <= 5 M tiles: one commit per tile
-            constexpr int ROUNDS = (G::END_TILES + 4) / 5;
-            static_assert(!TC || ROUNDS <= 2, "two mbarriers are reserved");
-            for (int r = 0; r < ROUNDS; ++r) mbar_init(smem_u32(bar_mma + r), (uint32_t)min(5, G::END_TILES - 5 * r));
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-        if (tid < 32) {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                         ::"r"(smem_u32(tmem_slot)), "r"(128u) : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-        }
-    }
-    if (!TMA) asm volatile("cp.async.wait_group 0;" ::: "memory");
     __syncthreads();
-    if (TMA) mbar_wait(smem_u32(bar), 0);
+    mbar_wait(smem_u32(bar), 0);
     hg_fold<NT>(sW + 2 * HG_WSLOT, sF);
     hg_fold<NT>(sW + 3 * HG_WSLOT, sF + 36);
     const int hy0 = oy0 / 2, hx0 = ox0 / 2, qy0 = oy0 / 4, qx0 = ox0 / 4;
     hg_down_pairs<G::D1H, G::D1W, G::D1P, G::XP, 5, NT>(sX, sD1, sW, hy0 - 6, hx0 - 6, p.H / 2, p.W / 2, p.alpha);
     __syncthreads();
-    if (TC) {                                            // the X block is dead: it now holds the `end` level's B operand
-        // B[ky][chunk c][n = phase][e]: k = 4 c + e is the float offset inside the A row; output column 4 pos + phase
-        // reads U1 columns 4 pos + phase + kx, i.e. weight w[ky][kx = k - phase]
-        for (int i = tid; i < G::END_B; i += NT) {
-            const int e = i & 3, n = (i >> 2) & 15, c = (i >> 6) & 1, ky = i >> 7;
-            const int kx = 4 * c + e - n;
-            sBend[i] = (n < 4 && kx >= 0 && kx < 5) ? round_tf32(__ldg(p.w[4] + ky * 5 + kx)) : 0.f;
-        }
-    }
     hg_down<G::D2H, G::D2W, G::D2P, G::D1P, (G::D2H % 2 == 0) ? 2 : 4, NT>(sD1, sD2, sW + HG_WSLOT, qy0 - 2, qx0 - 2, p.H / 4, p.W / 4, p.alpha);
     __syncthreads();
     hg_up<G::U2H, G::U2W, G::U2P, G::D2P, NT>(sD2, sU2, sF, sW[2 * HG_WSLOT + 25], hy0 - 2, hx0 - 2, p.H / 2, p.W / 2, p.alpha);
     __syncthreads();
-    hg_up<G::U1H, G::U1W, G::U1P, G::U2P, NT, TC>(sU2, sU1, sF + 36, sW[3 * HG_WSLOT + 25], oy0 - 2, ox0 - 2, p.H, p.W, p.alpha);
-    if (TC) {
-        // ---- end on the tensor core: y(r, 4 pos + ph) = act_end(b + sum_ky A_ky[m, :] . B_ky[:, ph]), m = r PPR + pos,
-        // A_ky[m, k] = U1 block float (r + ky) U1P + 4 pos + k: five tcgen05.mma (128 x 16 x 8, TF32) per M tile straight
-        // from the block in shared memory, FP32 accumulators in tensor memory, two rounds of <= 5 tiles (80 columns)
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");      // the block was written by the generic proxy
-        tc_fence_before();
-        __syncthreads();
-        tc_fence_after();
-        const uint32_t tmem = *tmem_slot;
-        const int warp = tid >> 5, lane = tid & 31;
-        const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((16u >> 3) << 17) | ((128u >> 4) << 24);
-        const float bias = sW[4 * HG_WSLOT + 25];
-        constexpr int ROUND = 5;
-        // descriptors in 16-byte units: + 128 per M tile (128 positions x 16 B), + U1P / 4 per kernel row; B: + 32 per
-        // kernel row (512 B).  One issuing lane per tile, spread over the CTA's warps: a single issuer would spend
-        // longer on the 45 MMAs' scalar bookkeeping than the FFMA version took for the whole level (measured).
-        const uint64_t da0 = make_kmajor_nosw_desc(smem_u32(sU1), 16, 128);
-        const uint64_t db0 = make_kmajor_nosw_desc(smem_u32(sBend), 256, 128);
-#pragma unroll 1
-        for (int t0 = 0, round = 0; t0 < G::END_TILES; t0 += ROUND, ++round) {
-            const int nt = min(ROUND, G::END_TILES - t0);
-            if (warp < nt) {
-                if (elect_one_hg()) {
-                    const uint64_t da = da0 + (uint64_t)((t0 + warp) * 128);
-                    const uint32_t d = tmem + 16u * (uint32_t)warp;
-#pragma unroll
-                    for (int ky = 0; ky < 5; ++ky)
-                        tc_mma_tf32(d, da + (uint64_t)(ky * (G::U1P / 4)), db0 + (uint64_t)(ky * 32), idesc, ky > 0);
-                    tc_commit(smem_u32(bar_mma + round));
-                }
-                __syncwarp();
-            }
-            mbar_wait(smem_u32(bar_mma + round), 0);
-            tc_fence_after();
-            // two warps per TMEM lane quarter: warp w and w + 4 take alternate tiles
-            for (int t = warp >> 2; t < nt; t += 2) {
-                uint32_t v[4];
-                asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"
-                             : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3])
-                             : "r"(tmem + ((uint32_t)((warp & 3) * 32) << 16) + 16u * t) : "memory");
-                tc_wait_ld();
-                const int m = (t0 + t) * 128 + (warp & 3) * 32 + lane;
-                const int r = m / G::PPR, c0 = 4 * (m - r * G::PPR);
-                const int gy = oy0 + r, gx = ox0 + c0;
-                if (r < TH && c0 < TW && gy < p.H && gx < p.W)            // W % 4 == 0: float4 granularity
-                    *reinterpret_cast<float4*>(yim + (int64_t)gy * p.W + gx) =
-                        make_float4(apply_act_fast(__uint_as_float(v[0]) + bias, p.act_end, p.alpha_end),
-                                    apply_act_fast(__uint_as_float(v[1]) + bias, p.act_end, p.alpha_end),
-                                    apply_act_fast(__uint_as_float(v[2]) + bias, p.act_end, p.alpha_end),
-                                    apply_act_fast(__uint_as_float(v[3]) + bias, p.act_end, p.alpha_end));
-            }
-            tc_fence_before();
-            __syncthreads();                                              // the accumulators are free for the next round
-            tc_fence_after();
-        }
-        if (tid < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(128u) : "memory");
-        return;
-    }
+    hg_up<G::U1H, G::U1W, G::U1P, G::U2P, NT>(sU2, sU1, sF + 36, sW[3 * HG_WSLOT + 25], oy0 - 2, ox0 - 2, p.H, p.W, p.alpha);
     __syncthreads();
     // ---- end: y(r, c) = act_end(conv5x5(U1)(r + ky, c + kx) + b); thread = 4 rows x 4 columns (16-byte loads at lane
     // stride: conflict-free; 8 input rows x 32 bytes per 16 outputs, was 6 x 32 per 8), one pass of the 256 threads
@@ -431,64 +305,51 @@ __global__ void __launch_bounds__(hg_threads(TH), TH >= 64 ? 2 : (TC ? 3 : 4)) h
     }
 }
 
-template <bool TMA, bool TC, int TH = 32>
-static int hourglass1_launch(const HourglassParams& p, const CUtensorMap& map, int64_t n, int64_t h, int64_t wd,
-                             cudaStream_t st) {
+static int hourglass1_unsupported() {
+    set_error("hourglass1_fwd: unsupported geometry (H, W must be multiples of 4)");
+    return UOCR_ERR_UNSUPPORTED;
+}
+
+template <int TH>
+static int hourglass1_launch(const HourglassParams& p, const float* x, int64_t n, int64_t h, int64_t wd, cudaStream_t st) {
     constexpr int TW = 128;
-    const size_t smem = sizeof(float) * (TC ? HG<TH, TW>::FLOATS_TC : HG<TH, TW>::FLOATS_ALIASED);
+    using G = HG<TH, TW>;
+    const uint64_t dims[3] = {(uint64_t)wd, (uint64_t)h, (uint64_t)n};
+    const uint64_t strides[2] = {(uint64_t)wd * 4, (uint64_t)wd * h * 4};
+    const uint32_t box[3] = {(uint32_t)G::XP, (uint32_t)G::XH, 1};
+    CUtensorMap map{};
+    const int rc = make_tmap_plain_f32(&map, x, 3, dims, strides, box);
+    if (rc != UOCR_OK) return rc;
+    const size_t smem = sizeof(float) * G::FLOATS;
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(hourglass1_fwd_kernel<TH, TW, TMA, TC>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(hourglass1_fwd_kernel<TH, TW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             (int)smem);
         if (e != cudaSuccess) { set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return UOCR_ERR_CUDA; }
         configured = true;
     }
     dim3 grid((unsigned)ceil_div(wd, TW), (unsigned)ceil_div(h, TH), (unsigned)n);
-    if (grid.y > 65535) return UOCR_ERR_UNSUPPORTED;
-    hourglass1_fwd_kernel<TH, TW, TMA, TC><<<grid, hg_threads(TH), smem, st>>>(p, map);
+    if (grid.y > 65535) return hourglass1_unsupported();
+    hourglass1_fwd_kernel<TH, TW><<<grid, hg_threads(TH), smem, st>>>(p, map);
     UOCR_LAUNCHED("hourglass1_fwd");
     return UOCR_OK;
 }
 
+// The kernel is the same in both math modes: its FFMA levels are exact FP32.  A tensor map that cannot be built
+// returns its own error and message.
 int hourglass1_fwd(const float* x, const float* const* w, const float* const* b, float* y, int64_t n, int64_t h,
-                   int64_t wd, float alpha, int act_end, float alpha_end, int math_mode, cudaStream_t st) {
-    if (h % 4 || wd % 4 || n > 65535 || alpha < 0.f || alpha > 1.f) return UOCR_ERR_UNSUPPORTED;
-    if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15) return UOCR_ERR_UNSUPPORTED;
+                   int64_t wd, float alpha, int act_end, float alpha_end, cudaStream_t st) {
+    if (h % 4 || wd % 4 || n > 65535 || alpha < 0.f || alpha > 1.f) return hourglass1_unsupported();
+    if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15) return hourglass1_unsupported();
     HourglassParams p{};
     p.x = x; p.y = y;
     for (int l = 0; l < 5; ++l) { p.w[l] = w[l]; p.b[l] = b[l]; }
     p.H = (int)h; p.W = (int)wd; p.alpha = alpha; p.act_end = act_end; p.alpha_end = alpha_end;
-    // UOCR_HOURGLASS_TMA=0: cp.async tile fill (the first version; kept for A/B runs)
-    const char* e = getenv("UOCR_HOURGLASS_TMA");
-    CUtensorMap map{};
-    if (!(e && e[0] == '0')) {
-        using G = HG<32, 128>;
-        const uint64_t dims[3] = {(uint64_t)wd, (uint64_t)h, (uint64_t)n};
-        const uint64_t strides[2] = {(uint64_t)wd * 4, (uint64_t)wd * h * 4};
-        // 64-row blocks with 512 threads where they still fill the machine twice over (2 CTAs / SM): 7 % fewer halo FMAs
-        // and half as many block prologues, 115.7 -> 111.6 us per 64 tiles.  UOCR_HOURGLASS_TH=32 / 64 forces either.
-        const char* th_env = getenv("UOCR_HOURGLASS_TH");
-        const int64_t blocks64 = n * ceil_div(h, 64) * ceil_div(wd, 128);
-        if (th_env ? atoi(th_env) == 64 : blocks64 >= 148 * 2 * 2) {
-            using G64 = HG<64, 128>;
-            const uint32_t box64[3] = {(uint32_t)G64::XP, (uint32_t)G64::XH, 1};
-            if (make_tmap_plain_f32(&map, x, 3, dims, strides, box64) == UOCR_OK)
-                return hourglass1_launch<true, false, 64>(p, map, n, h, wd, st);
-        }
-        const uint32_t box[3] = {(uint32_t)G::XP, (uint32_t)G::XH, 1};
-        if (make_tmap_plain_f32(&map, x, 3, dims, strides, box) == UOCR_OK) {
-            // UOCR_HOURGLASS_TC=1 (TF32 mode only): the full-resolution `end` level as tcgen05.mma straight from the U1
-            // block in shared memory.  A measured NEGATIVE result, off by default: 150 us per 64 tiles against 123 us
-            // for the FFMA level.  The kernel is bound by shared-memory bandwidth (L1 / shared pipe 77 % busy), and the
-            // MMA's A operand re-reads the block once per kernel row (5 x 32 B per 4 outputs = 40 B per output) where
-            // the FFMA level's 2 x 4 register tiles read 24 B per output; sharing A rows between output rows would
-            // need M tiles that do not cross image rows, i.e. 34 of 128 lanes used at this block width.
-            const char* tc = getenv("UOCR_HOURGLASS_TC");
-            if (math_mode == UOCR_MATH_TF32 && tc && tc[0] == '1') return hourglass1_launch<true, true>(p, map, n, h, wd, st);
-            return hourglass1_launch<true, false>(p, map, n, h, wd, st);
-        }
-    }
-    return hourglass1_launch<false, false>(p, map, n, h, wd, st);
+    // 64-row blocks with 512 threads where they still fill the machine twice over (2 CTAs / SM): 7 % fewer halo FMAs
+    // and half as many block prologues, 115.7 -> 111.6 us per 64 tiles.
+    const int64_t blocks64 = n * ceil_div(h, 64) * ceil_div(wd, 128);
+    if (blocks64 >= 148 * 2 * 2) return hourglass1_launch<64>(p, x, n, h, wd, st);
+    return hourglass1_launch<32>(p, x, n, h, wd, st);
 }
 
 }  // namespace uocr
@@ -501,9 +362,7 @@ static int hourglass1_entry(const float* x, const float* const* weights, const f
     UOCR_REQUIRE(n > 0 && h > 0 && w > 0 && h < (1 << 30) && w < (1 << 30), "bad dimension");
     UOCR_REQUIRE(act_end >= UOCR_ACT_NONE && act_end <= UOCR_ACT_SIGMOID, "unknown activation %d", act_end);
     UOCR_REQUIRE(math_mode == UOCR_MATH_FP32 || math_mode == UOCR_MATH_TF32, "unknown math mode %d", math_mode);
-    const int rc = hourglass1_fwd(x, weights, biases, y, n, h, w, alpha, act_end, alpha_end, math_mode, as_stream(stream));
-    if (rc == UOCR_ERR_UNSUPPORTED) set_error("hourglass1_fwd: unsupported geometry (H, W must be multiples of 4)");
-    return rc;
+    return hourglass1_fwd(x, weights, biases, y, n, h, w, alpha, act_end, alpha_end, as_stream(stream));
 }
 
 extern "C" int uocr_hourglass1_fwd(const float* x, const float* const* weights, const float* const* biases, float* y,

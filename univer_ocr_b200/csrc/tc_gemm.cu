@@ -52,62 +52,43 @@ static EncodeTiledFn encode_tiled() {
     return fn;
 }
 
-static CUtensorMapDataType tmap_dtype() {
-    static int mode = -1;
-    if (mode < 0) {
-        const char* e = getenv("UOCR_TMA_DTYPE");          // "f32" = raw bits (tensor core truncates)
-        mode = (e && e[0] == 'f') ? 0 : 1;
-    }
-    return mode ? CU_TENSOR_MAP_DATA_TYPE_TFLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
-}
-
-// rank-`rank` fp32 tensor, dims innermost first, 128-byte swizzled boxes
-static int make_tmap(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
-                     const uint64_t* strides_bytes /* rank-1 */, const uint32_t* box, bool mn_major = false) {
+// rank-`rank` fp32 tensor, dims innermost first.  The three flavours differ only in data type, swizzle and L2 promotion.
+static int encode_tmap(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
+                       const uint64_t* strides_bytes /* rank-1 */, const uint32_t* box, CUtensorMapDataType dtype,
+                       CUtensorMapSwizzle swizzle, CUtensorMapL2promotion l2) {
     EncodeTiledFn fn = encode_tiled();
     if (!fn) { set_error("cuTensorMapEncodeTiled is unavailable"); return UOCR_ERR_UNSUPPORTED; }
     cuuint64_t gd[5]; cuuint64_t gs[4]; cuuint32_t bx[5]; cuuint32_t es[5];
     for (int i = 0; i < rank; ++i) { gd[i] = dims[i]; bx[i] = box[i]; es[i] = 1; }
     for (int i = 0; i + 1 < rank; ++i) gs[i] = strides_bytes[i];
-    CUresult r = fn(map, tmap_dtype(), (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE,
-                    // MN-major 32-bit operands must use the 32-byte-atom flavour of the 128B swizzle
-                    // (UMMA layout SWIZZLE_128B_BASE32B); K-major operands the plain 16-byte one
-                    mn_major ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B,
-                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    CUresult r = fn(map, dtype, (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                    swizzle, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed (%d)", (int)r); return UOCR_ERR_UNSUPPORTED; }
     return UOCR_OK;
+}
+
+// 128-byte swizzled tcgen05 operand boxes, rounded to TF32 by the TMA unit.  MN-major 32-bit operands must use the
+// 32-byte-atom flavour of the 128B swizzle (UMMA layout SWIZZLE_128B_BASE32B); K-major operands the plain 16-byte one.
+static int make_tmap(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
+                     const uint64_t* strides_bytes /* rank-1 */, const uint32_t* box, bool mn_major = false) {
+    return encode_tmap(map, base, rank, dims, strides_bytes, box, CU_TENSOR_MAP_DATA_TYPE_TFLOAT32,
+                       mn_major ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B,
+                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
 }
 
 // plain (no swizzle, raw FP32) boxes: kernels that stage an image block for the CUDA cores (hourglass.cu)
 int make_tmap_plain_f32(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
                         const uint64_t* strides_bytes /* rank-1 */, const uint32_t* box) {
-    EncodeTiledFn fn = encode_tiled();
-    if (!fn) { set_error("cuTensorMapEncodeTiled is unavailable"); return UOCR_ERR_UNSUPPORTED; }
-    cuuint64_t gd[5]; cuuint64_t gs[4]; cuuint32_t bx[5]; cuuint32_t es[5];
-    for (int i = 0; i < rank; ++i) { gd[i] = dims[i]; bx[i] = box[i]; es[i] = 1; }
-    for (int i = 0; i + 1 < rank; ++i) gs[i] = strides_bytes[i];
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled (plain) failed (%d)", (int)r); return UOCR_ERR_UNSUPPORTED; }
-    return UOCR_OK;
+    return encode_tmap(map, base, rank, dims, strides_bytes, box, CU_TENSOR_MAP_DATA_TYPE_FLOAT32,
+                       CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
 }
 
 // plain (no swizzle) boxes whose elements the TMA unit rounds to TF32 (round to nearest): image rows that a tcgen05.mma
 // reads directly as its A operand (conv_pair_rows_tc.cu)
 int make_tmap_plain_tf32(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
                          const uint64_t* strides_bytes /* rank-1 */, const uint32_t* box) {
-    EncodeTiledFn fn = encode_tiled();
-    if (!fn) { set_error("cuTensorMapEncodeTiled is unavailable"); return UOCR_ERR_UNSUPPORTED; }
-    cuuint64_t gd[5]; cuuint64_t gs[4]; cuuint32_t bx[5]; cuuint32_t es[5];
-    for (int i = 0; i < rank; ++i) { gd[i] = dims[i]; bx[i] = box[i]; es[i] = 1; }
-    for (int i = 0; i + 1 < rank; ++i) gs[i] = strides_bytes[i];
-    CUresult r = fn(map, tmap_dtype(), (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled (plain tf32) failed (%d)", (int)r); return UOCR_ERR_UNSUPPORTED; }
-    return UOCR_OK;
+    return encode_tmap(map, base, rank, dims, strides_bytes, box, CU_TENSOR_MAP_DATA_TYPE_TFLOAT32,
+                       CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
 }
 
 constexpr int TC_BM = 128;           // UMMA M
@@ -371,17 +352,11 @@ __global__ void __launch_bounds__(TC_THREADS, 2) tc_gemm_kernel(const __grid_con
     }
 }
 
-static int env_int(const char* name, int fallback) {
-    const char* e = getenv(name);
-    return e ? atoi(e) : fallback;
-}
-
 static int pick_stages(int nt, size_t* smem_bytes) {
     const size_t a_bytes = TC_BM * TC_BK * 4;
     const size_t b_bytes = (((size_t)nt * TC_BK * 4) + 1023) & ~(size_t)1023;
-    static const int budget_kb = env_int("UOCR_TC_SMEM_KB", 70);     // ~3 CTAs / SM: their prologues and
-                                                                       // epilogues overlap other CTAs' main loops
-    const size_t budget = (size_t)budget_kb * 1024;
+    // 70 KB: ~3 CTAs / SM, so that their prologues and epilogues overlap other CTAs' main loops
+    const size_t budget = (size_t)70 * 1024;
     int stages = (int)((budget - 2048) / (a_bytes + b_bytes));
     if (stages > 8) stages = 8;
     if (stages < 2) stages = 2;
@@ -406,8 +381,7 @@ static int launch_tc(const CUtensorMap& ma, const CUtensorMap& mb, TcParams& p, 
 }
 
 static int pick_nt(int64_t n) {
-    static const int cap = env_int("UOCR_TC_NT", 64);
-    if (n >= cap) return cap;                 // full-rate N; wider tiles amortise the A reads
+    if (n >= 64) return 64;                   // full-rate N; wider tiles amortise the A reads
     return (int)(((n + 15) / 16) * 16);
 }
 
@@ -422,11 +396,9 @@ int tc_gemm_tn(const float* A, int64_t lda, const float* Bt, int64_t ldb, float*
         return UOCR_ERR_UNSUPPORTED;            // TMA: 16-byte aligned base and row pitch
     if (M <= 0 || N <= 0 || K <= 0 || M > 0x7fffffff || K > 0x7fffffff) return UOCR_ERR_UNSUPPORTED;
     {
-        // enough 128 x NT tiles to keep most SMs busy (dense_2: 128 tiles, 46 -> 34 us)
-        static const int persist = env_int("UOCR_TC_PERSISTENT", 1);
+        // enough 128 x NT tiles to keep most SMs busy (dense_2: 128 tiles, 46 -> 34 us): >= 96, ~2/3 of the SMs
         const int64_t nt = N >= 256 ? 256 : ((N + 15) / 16) * 16;
-        static const int min_tiles = env_int("UOCR_TC_PERSISTENT_MIN_TILES", 96);   // >= ~2/3 of the SMs busy
-        if (persist && N >= 128 && ceil_div(M, TC_BM) * ceil_div(N, nt) >= min_tiles) {
+        if (N >= 128 && ceil_div(M, TC_BM) * ceil_div(N, nt) >= 96) {
             const int rc = tc_gemm_tn_persistent(A, lda, Bt, ldb, C, ldc, M, N, K, bias, act, alpha, accumulate, st);
             if (rc != UOCR_ERR_UNSUPPORTED) return rc;
         }
@@ -814,8 +786,7 @@ int tc_gemm_mn_atomic(const float* At, int64_t lda, const float* B, int64_t ldb,
     // Char head's weight gradients (tools/trainprof.py): dense_1 0.185 -> 0.149 ms, dense_2 0.105 -> 0.097, dense_3
     // (one tile, 128-way contention) 0.085 -> 0.071
     int64_t splits = (148 + tiles - 1) / tiles;
-    static const int min_kb = env_int("UOCR_TC_WGRAD_MIN_KB", 8);
-    if (splits > p.num_kb / min_kb) splits = p.num_kb / min_kb;
+    if (splits > p.num_kb / 8) splits = p.num_kb / 8;
     if (splits < 1) splits = 1;
     if (splits > 65535) splits = 65535;
     p.kb_per_split = (int)ceil_div(p.num_kb, splits);
@@ -1071,43 +1042,31 @@ int conv_fwd_tc(const ConvGeom& g, const float* x, const float* w, const float* 
 // Convolutional2D forward, slab variant (Char conv_2 / conv_3: 5x3, 64 -> 64, stride (2, 1)).
 // ncu on the one-tile-per-CTA kernel above: every (ky, kx, channel block) step re-fetches a 16 KB A tile and an
 // 8 KB B tile from L2 -- 720 KB per 128-pixel tile, 460 MB through L2 for a 59 MB input, i.e. L2 -> SM bandwidth
-// bound at 20 % of the tensor peak.  Here a pipeline stage holds, for one (ky, channel block),
-//   * XB input-row SLABS of 128 + kw - 1 pixels x 32 channels (one per 128-pixel x-block of the output row): the
-//     kw horizontal taps are the SAME slab read from a start address shifted by kx pixel rows (128 B each; the
-//     128-byte swizzle is a function of the absolute shared-memory address, so a start address that is not
-//     1024-byte aligned needs nothing else -- setting the descriptor's base-offset field to the row phase gives
-//     wrong results, tested), so A is fetched once per kernel ROW instead of once per tap, and
-//   * the kw weight chunks of that kernel row, shared by the XB x-blocks (two accumulators in TMEM).
+// bound at 20 % of the tensor peak.  Here a CTA owns one 128-pixel x-block of one output row, and a pipeline stage
+// holds, for one (ky, channel block),
+//   * an input-row SLAB of 128 + kw - 1 pixels x 32 channels: the kw horizontal taps are the SAME slab read from a
+//     start address shifted by kx pixel rows (128 B each; the 128-byte swizzle is a function of the absolute
+//     shared-memory address, so a start address that is not 1024-byte aligned needs nothing else -- setting the
+//     descriptor's base-offset field to the row phase gives wrong results, tested), so A is fetched once per kernel
+//     ROW instead of once per tap, and
+//   * the kw weight chunks of that kernel row.
 // Per 128-pixel tile that is 286 KB instead of 720 KB through L2.
 // ------------------------------------------------------------------------------------------
 struct SlabParams {
     float* y; const float* bias;
     int n_img, ho, wo, cout, nt;
     int kh, kw, sh, ph, pw, cblocks;
-    int xb;                           // x-blocks per CTA (1 or 2)
     int stages;
     uint32_t slab_bytes, slab_box_bytes, b_bytes;
     int act; float alpha;
-    int base_offset_mode;             // 1: descriptor base offset = row phase of the start address
 };
 
-__device__ __forceinline__ uint64_t make_kmajor_sw128_desc_off(uint32_t smem_addr, int with_base_offset) {
-    uint64_t d = make_kmajor_sw128_desc(smem_addr);
-    if (with_base_offset == 1) d |= (uint64_t)((smem_addr >> 7) & 7u) << 49;
-    return d;
-}
-
-// MC: the two CTAs of a cluster are the two x-blocks of one output row.  They need the same weight chunks, so each
-// fetches HALF of every chunk (cout / 2 rows, map_b's box) and multicasts it to both; a stage is refilled only when the
-// MMAs of BOTH CTAs have released it (empty[] counts 2, the commits are multicast).  Halves the weight traffic through
-// L2, which was 57 % of this kernel's operand bytes.
-template <bool MC>
 __global__ void __launch_bounds__(TC_THREADS, 1) tc_conv_slab_kernel(const __grid_constant__ CUtensorMap map_a,
                                                                      const __grid_constant__ CUtensorMap map_b,
                                                                      const SlabParams p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    const uint32_t stage_bytes = (uint32_t)p.xb * p.slab_bytes + (uint32_t)p.kw * p.b_bytes;
+    const uint32_t stage_bytes = p.slab_bytes + (uint32_t)p.kw * p.b_bytes;
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)p.stages * stage_bytes);
     uint64_t* full = bars;
     uint64_t* empty = bars + p.stages;
@@ -1116,16 +1075,15 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_conv_slab_kernel(const __gri
     float* s_bias = reinterpret_cast<float*>(bars + 2 * p.stages + 2);      // nt floats (zeros without a bias)
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     for (int i = threadIdx.x; i < p.nt; i += TC_THREADS) s_bias[i] = (p.bias && i < p.cout) ? __ldg(p.bias + i) : 0.f;
-    const int cx_base = blockIdx.x * p.xb * TC_BM, oy = blockIdx.y, cn = blockIdx.z;
-    const int xb_live = min(p.xb, (p.wo - cx_base + TC_BM - 1) / TC_BM);       // x-blocks inside the row
+    const int cx = blockIdx.x * TC_BM, oy = blockIdx.y, cn = blockIdx.z;
     const int num_it = p.kh * p.cblocks;
     uint32_t tmem_cols = 32;
-    while ((int)tmem_cols < p.xb * p.nt) tmem_cols <<= 1;
+    while ((int)tmem_cols < p.nt) tmem_cols <<= 1;
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < p.stages; ++s) {
             mbar_init(smem_u32(&full[s]), 1);
-            mbar_init(smem_u32(&empty[s]), MC ? 2 : 1);
+            mbar_init(smem_u32(&empty[s]), 1);
         }
         mbar_init(smem_u32(tmem_full), 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -1136,11 +1094,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_conv_slab_kernel(const __gri
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     tc_fence_before();
-    if (MC) cluster_sync_all();             // the peer's barriers exist before anything is multicast to them
-    else __syncthreads();
+    __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    const uint32_t rank = MC ? cluster_ctarank() : 0u;
 
     if (warp == 0) {
         if (lane == 0) {
@@ -1149,19 +1105,13 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_conv_slab_kernel(const __gri
                 mbar_wait(smem_u32(&empty[s]), ((it / p.stages) & 1) ^ 1);
                 const int ky = it / p.cblocks, cb = it - ky * p.cblocks;
                 const uint32_t sa = smem_u32(smem + (size_t)s * stage_bytes);
-                const uint32_t sb = sa + (uint32_t)p.xb * p.slab_bytes;
+                const uint32_t sb = sa + p.slab_bytes;
                 const uint32_t bar = smem_u32(&full[s]);
-                mbar_arrive_expect_tx(bar, (uint32_t)xb_live * p.slab_box_bytes + (uint32_t)p.kw * p.b_bytes);
-                for (int xb = 0; xb < xb_live; ++xb)
-                    tma_load_4d(sa + (uint32_t)xb * p.slab_bytes, &map_a, bar, cb * TC_BK, cx_base + xb * TC_BM - p.pw,
-                                oy * p.sh + ky - p.ph, cn);
+                mbar_arrive_expect_tx(bar, p.slab_box_bytes + (uint32_t)p.kw * p.b_bytes);
+                tma_load_4d(sa, &map_a, bar, cb * TC_BK, cx - p.pw, oy * p.sh + ky - p.ph, cn);
                 for (int kx = 0; kx < p.kw; ++kx) {
                     const int k0 = ((ky * p.kw + kx) * p.cblocks + cb) * TC_BK;
-                    if (MC)                  // rows [rank * cout / 2, ..) of the chunk, to both CTAs
-                        tma_load_2d_mc(sb + (uint32_t)kx * p.b_bytes + rank * (p.b_bytes / 2), &map_b, bar, k0,
-                                       (int)rank * (p.nt / 2), (uint16_t)3);
-                    else
-                        tma_load_2d(sb + (uint32_t)kx * p.b_bytes, &map_b, bar, k0, 0);
+                    tma_load_2d(sb + (uint32_t)kx * p.b_bytes, &map_b, bar, k0, 0);
                 }
             }
         }
@@ -1174,20 +1124,17 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_conv_slab_kernel(const __gri
                 mbar_wait(smem_u32(&full[s]), (it / p.stages) & 1);
                 tc_fence_after();
                 const uint32_t sa = smem_u32(smem + (size_t)s * stage_bytes);
-                const uint32_t sb = sa + (uint32_t)p.xb * p.slab_bytes;
-                for (int xb = 0; xb < xb_live; ++xb)
-                    for (int kx = 0; kx < p.kw; ++kx) {
-                        // the tap's A operand = the slab from pixel row kx on
-                        const uint64_t da = make_kmajor_sw128_desc_off(sa + (uint32_t)xb * p.slab_bytes + (uint32_t)kx * (p.base_offset_mode == 3 ? 0u : 128u),
-                                                                       p.base_offset_mode);
-                        const uint64_t db = make_kmajor_sw128_desc(sb + (uint32_t)kx * p.b_bytes);
+                const uint32_t sb = sa + p.slab_bytes;
+                for (int kx = 0; kx < p.kw; ++kx) {
+                    // the tap's A operand = the slab from pixel row kx on
+                    const uint64_t da = make_kmajor_sw128_desc(sa + (uint32_t)kx * 128u);
+                    const uint64_t db = make_kmajor_sw128_desc(sb + (uint32_t)kx * p.b_bytes);
 #pragma unroll
-                        for (int k = 0; k < TC_BK / 8; ++k)
-                            tc_mma_tf32(tmem_base + (uint32_t)(xb * p.nt), da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc,
-                                        (it > 0 || kx > 0 || k > 0) ? 1u : 0u);
-                    }
-                if (MC) tc_commit_mc(smem_u32(&empty[s]), (uint16_t)3);
-                else tc_commit(smem_u32(&empty[s]));
+                    for (int k = 0; k < TC_BK / 8; ++k)
+                        tc_mma_tf32(tmem_base, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc,
+                                    (it > 0 || kx > 0 || k > 0) ? 1u : 0u);
+                }
+                tc_commit(smem_u32(&empty[s]));
             }
             tc_commit(smem_u32(tmem_full));
         }
@@ -1195,32 +1142,29 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_conv_slab_kernel(const __gri
         const int q = warp & 3;
         mbar_wait(smem_u32(tmem_full), 0);
         tc_fence_after();
-        for (int xb = 0; xb < xb_live; ++xb) {
-            const int ox = cx_base + xb * TC_BM + q * 32 + lane;
-            float* dst = p.y + (((int64_t)cn * p.ho + oy) * p.wo + ox) * p.cout;
-            for (int c0 = 0; c0 < p.nt; c0 += 32) {
-                float v[32];
-                tc_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(xb * p.nt + c0), v);
-                if (ox >= p.wo) continue;
-                const float4* bs = reinterpret_cast<const float4*>(s_bias + c0);
+        const int ox = cx + q * 32 + lane;
+        float* dst = p.y + (((int64_t)cn * p.ho + oy) * p.wo + ox) * p.cout;
+        for (int c0 = 0; c0 < p.nt; c0 += 32) {
+            float v[32];
+            tc_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, v);
+            if (ox >= p.wo) continue;
+            const float4* bs = reinterpret_cast<const float4*>(s_bias + c0);
 #pragma unroll
-                for (int j = 0; j < 32; j += 4) {
-                    if (c0 + j < p.cout) {                                   // cout % 16 == 0
-                        const float4 b4 = bs[j >> 2];
-                        float4 o;
-                        o.x = apply_act_fast(v[j] + b4.x, p.act, p.alpha);
-                        o.y = apply_act_fast(v[j + 1] + b4.y, p.act, p.alpha);
-                        o.z = apply_act_fast(v[j + 2] + b4.z, p.act, p.alpha);
-                        o.w = apply_act_fast(v[j + 3] + b4.w, p.act, p.alpha);
-                        *reinterpret_cast<float4*>(dst + c0 + j) = o;
-                    }
+            for (int j = 0; j < 32; j += 4) {
+                if (c0 + j < p.cout) {                                   // cout % 16 == 0
+                    const float4 b4 = bs[j >> 2];
+                    float4 o;
+                    o.x = apply_act_fast(v[j] + b4.x, p.act, p.alpha);
+                    o.y = apply_act_fast(v[j + 1] + b4.y, p.act, p.alpha);
+                    o.z = apply_act_fast(v[j + 2] + b4.z, p.act, p.alpha);
+                    o.w = apply_act_fast(v[j + 3] + b4.w, p.act, p.alpha);
+                    *reinterpret_cast<float4*>(dst + c0 + j) = o;
                 }
             }
         }
     }
     tc_fence_before();
-    if (MC) cluster_sync_all();             // the peer's last commits arrive on this CTA's barriers: do not exit before them
-    else __syncthreads();
+    __syncthreads();
     if (warp == 1) {
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(tmem_cols) : "memory");
@@ -1229,31 +1173,24 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_conv_slab_kernel(const __gri
 
 static int conv_fwd_tc_slab(const ConvGeom& g, const float* x, const float* wt /* (Cout, K) */, const float* b, float* y,
                             int act, float alpha, cudaStream_t st) {
-    static const int mode = env_int("UOCR_CONV_SLAB", 2);          // 0: off; 2: plain descriptors (correct: the swizzle is a
-                                                                   // function of the absolute smem address); 1: with the row phase in
-                                                                   // the base-offset field -- measured WRONG results, kept for the record
-    if (!mode || g.kw > 8 || g.cout > 128 || (reinterpret_cast<uintptr_t>(y) & 15)) return UOCR_ERR_UNSUPPORTED;
+    if (g.kw > 8 || g.cout > 128 || (reinterpret_cast<uintptr_t>(y) & 15)) return UOCR_ERR_UNSUPPORTED;
     if (g.n > 65535 || g.ho > 65535) return UOCR_ERR_UNSUPPORTED;
     SlabParams p{};
     p.y = y; p.bias = g.bias ? b : nullptr;
     p.n_img = g.n; p.ho = g.ho; p.wo = g.wo; p.cout = g.cout; p.nt = g.cout;
     p.kh = g.kh; p.kw = g.kw; p.sh = g.sh; p.ph = g.ph; p.pw = g.pw; p.cblocks = g.cin / TC_BK;
-    p.act = act; p.alpha = alpha; p.base_offset_mode = mode == 1 ? 1 : (mode == 3 ? 3 : 0);
+    p.act = act; p.alpha = alpha;
     const int xtiles = (g.wo + TC_BM - 1) / TC_BM;
-    // Measured on Char conv_2 (64 tiles of 5 x 256 pixels): 1 x-block + 2 stages (84 KB: two CTAs per SM, so one
-    // CTA's prologue / epilogue overlaps the other's main loop) 0.050 ms; 2 x-blocks sharing B with 3 stages (one CTA
-    // per SM) 0.067 ms; the one-tile-per-CTA kernel 0.065 ms.  UOCR_CONV_SLAB_XB / _STAGES override.
-    static const int xb_env = env_int("UOCR_CONV_SLAB_XB", 1);
-    p.xb = xb_env == 2 && xtiles >= 2 ? 2 : 1;
-    static const int max_stages = env_int("UOCR_CONV_SLAB_STAGES", 2);
-    static const int box_round = env_int("UOCR_CONV_SLAB_BOXROUND", 1);
-    const uint32_t box_rows = box_round > 1 ? ((TC_BM + g.kw - 1 + box_round - 1) / box_round) * box_round : TC_BM + g.kw - 1;
+    // Measured on Char conv_2 (64 tiles of 5 x 256 pixels): 2 stages (84 KB: two CTAs per SM, so one CTA's prologue /
+    // epilogue overlaps the other's main loop) 0.050 ms; 2 x-blocks per CTA sharing B with 3 stages (one CTA per SM)
+    // 0.067 ms; the one-tile-per-CTA kernel 0.065 ms.
+    const uint32_t box_rows = TC_BM + g.kw - 1;
     p.slab_box_bytes = box_rows * 128u;
     p.slab_bytes = (p.slab_box_bytes + 1023u) & ~1023u;
     p.b_bytes = (uint32_t)g.cout * 128u;                            // cout % 16 == 0 -> multiple of 2048: 1024-aligned
-    const uint32_t stage_bytes = (uint32_t)p.xb * p.slab_bytes + (uint32_t)g.kw * p.b_bytes;
+    const uint32_t stage_bytes = p.slab_bytes + (uint32_t)g.kw * p.b_bytes;
     p.stages = (int)((200u * 1024u) / stage_bytes);
-    if (p.stages > max_stages) p.stages = max_stages;
+    if (p.stages > 2) p.stages = 2;
     if (p.stages < 2 || (p.b_bytes & 1023u)) return UOCR_ERR_UNSUPPORTED;
     const size_t smem = (size_t)p.stages * stage_bytes + 1024 + (2 * p.stages + 2) * 8 + 4 * 128 + 64;
     const int K = g.kh * g.kw * g.cin;
@@ -1263,38 +1200,18 @@ static int conv_fwd_tc_slab(const ConvGeom& g, const float* x, const float* wt /
     const uint32_t ba[4] = {TC_BK, box_rows, 1, 1};
     int rc = make_tmap(&ma, x, 4, da, sa, ba);
     if (rc) return rc;
-    // UOCR_CONV_SLAB_MC=1: two x-blocks per output row (Char: wo = 256) run as a cluster and share the weight fetches by
-    // TMA multicast.  A measured NEGATIVE result, off by default: conv_2 44.7 -> 48.5 us, the step 0.379 -> 0.386 ms.
-    // Halving the weight traffic through L2 (57 % of the operand bytes) buys nothing because the kernel is not held up by
-    // L2 bytes but by per-CTA latency at 2 stages, and the shared stages make the two CTAs of a cluster wait for each
-    // other (a stage is refilled only when both have released it).
-    const int mc_env = env_int("UOCR_CONV_SLAB_MC", 0);
-    const bool mc = mc_env && p.xb == 1 && xtiles == 2 && g.wo == 2 * TC_BM && (p.b_bytes / 2) % 1024 == 0;
     const uint64_t db[2] = {(uint64_t)K, (uint64_t)g.cout}, sb[1] = {(uint64_t)K * 4};
-    const uint32_t bb[2] = {TC_BK, (uint32_t)(mc ? g.cout / 2 : g.cout)};
+    const uint32_t bb[2] = {TC_BK, (uint32_t)g.cout};
     rc = make_tmap(&mb, wt, 2, db, sb, bb);
     if (rc) return rc;
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(tc_conv_slab_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(tc_conv_slab_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaError_t e = cudaFuncSetAttribute(tc_conv_slab_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         if (e != cudaSuccess) { set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return UOCR_ERR_CUDA; }
         configured = true;
     }
-    dim3 grid((unsigned)ceil_div(xtiles, p.xb), (unsigned)g.ho, (unsigned)g.n);
-    if (mc) {
-        cudaLaunchConfig_t cfg{};
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.gridDim = grid; cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-        cfg.attrs = attr; cfg.numAttrs = 1;
-        cudaError_t e = cudaLaunchKernelEx(&cfg, tc_conv_slab_kernel<true>, ma, mb, p);
-        if (e != cudaSuccess) { set_error("cluster launch: %s", cudaGetErrorString(e)); return UOCR_ERR_CUDA; }
-    } else {
-        tc_conv_slab_kernel<false><<<grid, TC_THREADS, smem, st>>>(ma, mb, p);
-    }
+    dim3 grid((unsigned)xtiles, (unsigned)g.ho, (unsigned)g.n);
+    tc_conv_slab_kernel<<<grid, TC_THREADS, smem, st>>>(ma, mb, p);
     UOCR_LAUNCHED("tc_conv_slab_tf32");
     return UOCR_OK;
 }
@@ -1377,190 +1294,6 @@ int conv_wgrad_tc(const ConvGeom& g, const float* x, const float* dy, float* dw,
         cudaError_t e = cudaMemsetAsync(db, 0, sizeof(float) * g.cout, st);
         if (e != cudaSuccess) { set_error("memset: %s", cudaGetErrorString(e)); return UOCR_ERR_CUDA; }
     }
-    return UOCR_OK;
-}
-
-// ------------------------------------------------------------------------------------------
-// Monochrome pair on tensor cores: y = act2(conv3x3(act1(conv3x3(x, w1) + b1), w2) + b2),
-// 1 -> 16 -> 1 channels (my_model/model.py:119-122), inference.
-//
-// The 16 -> 1 convolution holds half of the pair's 288 FMA / pixel.  As an implicit GEMM it is
-// M = 128 pixels of one output row, K = 9 taps x 16 channels, N = 1 (padded to the minimum UMMA
-// N = 16): 18 tcgen05.mma (128x16x8, 8 cycles each) per 128 pixels instead of 128 x 144 FFMA.
-// The CTA first evaluates the hidden tile ((TH+2) x 130 pixels x 16 channels) on the CUDA cores and
-// stores it in shared memory as four channel-quad PLANES of 16-byte pixel entries -- the K-major
-// no-swizzle canonical layout with a pixel stride of 16 B, so that "8 rows" are always 128
-// contiguous bytes (SBO = 128) and the channel quads are LBO = one plane apart.  Because the
-// layout is linear in the pixel index, the A operand of kernel tap (ky, kx) for output row r is the
-// SAME buffer addressed from pixel ((r + ky) * 130 + kx): no im2col copy, just a start address.
-// One accumulator (16 TMEM columns, column 0 meaningful) per output row; the epilogue reads
-// column 0 with tcgen05.ld.32x32b.x1 -- lane = pixel, so the stores are fully coalesced.
-// ------------------------------------------------------------------------------------------
-constexpr int PT_TH = 8;             // output rows per CTA
-constexpr int PT_TW = 128;           // output columns per CTA = UMMA M
-constexpr int PT_HP = PT_TW + 2;     // hidden tile width
-constexpr int PT_XP = 136;           // x tile pitch (>= PT_TW + 4)
-constexpr int PT_C1 = 16;
-constexpr int PT_PLANE = (PT_TH + 2) * PT_HP * 16;    // bytes per channel-quad plane
-
-
-
-constexpr int PT_THREADS = 288;      // warps 0-7: hidden tile + epilogue; warp 8: hidden tile + MMA issue
-
-__global__ void __launch_bounds__(PT_THREADS, 2) conv3x3_pair_tc_kernel(
-    const float* __restrict__ x, const float* __restrict__ w1, const float* __restrict__ b1,
-    const float* __restrict__ w2, const float* __restrict__ b2, float* __restrict__ y, int H, int W, int act1,
-    float alpha1, int act2, float alpha2) {
-    extern __shared__ __align__(128) uint8_t pt_smem[];
-    float* s_h = reinterpret_cast<float*>(pt_smem);                                  // 4 planes
-    float* s_b = reinterpret_cast<float*>(pt_smem + 4 * PT_PLANE);                   // 36 chunks x 256 B
-    float* s_x = s_b + 36 * 64;                                                      // (TH+4) x XP
-    float* s_w1 = s_x + (PT_TH + 4) * PT_XP;                                         // 9*16 + 16
-    uint64_t* bar = reinterpret_cast<uint64_t*>(s_w1 + 160);
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar + 1);
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int x0 = blockIdx.x * PT_TW, y0 = blockIdx.y * PT_TH;
-    const float* xim = x + (int64_t)blockIdx.z * H * W;
-    float* yim = y + (int64_t)blockIdx.z * H * W;
-
-    // ---- phase 0: stage x tile, weights, the B operand; allocate TMEM
-    for (int i = tid; i < (PT_TH + 4) * PT_XP; i += PT_THREADS) {
-        const int r = i / PT_XP, c = i - r * PT_XP;
-        const int gy = y0 - 2 + r, gx = x0 - 2 + c;
-        s_x[i] = (gy >= 0 && gy < H && gx >= 0 && gx < W) ? __ldg(xim + (int64_t)gy * W + gx) : 0.f;
-    }
-    for (int i = tid; i < 160; i += PT_THREADS) s_w1[i] = i < 144 ? w1[i] : b1[i - 144];
-    for (int i = tid; i < 36 * 64; i += PT_THREADS) {
-        // chunk q = tap * 4 + quad; 64 floats per chunk = 16 rows (n) x 4 floats; only n == 0 is real
-        const int q = i >> 6, within = i & 63;
-        s_b[i] = within < 4 ? round_tf32(w2[(q >> 2) * PT_C1 + (q & 3) * 4 + within]) : 0.f;
-    }
-    if (tid == 0) {
-        mbar_init(smem_u32(bar), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    constexpr uint32_t TMEM_COLS = PT_TH * 16;          // 128
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                     ::"r"(smem_u32(tmem_slot)), "r"(TMEM_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-    // ---- phase 1: hidden tile on the CUDA cores; work item = (strip of 5 pixels, channel quad)
-    constexpr int STRIPS_PER_ROW = PT_HP / 5;           // 26
-    for (int item = tid; item < (PT_TH + 2) * STRIPS_PER_ROW * 4; item += PT_THREADS) {
-        const int quad = item & 3, s = item >> 2;
-        const int r = s / STRIPS_PER_ROW, c0 = (s - r * STRIPS_PER_ROW) * 5;
-        const int hy = y0 - 1 + r;
-        float xw[3][7];
-#pragma unroll
-        for (int a = 0; a < 3; ++a)
-#pragma unroll
-            for (int b = 0; b < 7; ++b) xw[a][b] = s_x[(r + a) * PT_XP + c0 + b];
-        const bool row_in = hy >= 0 && hy < H;
-        const float4 bq = *reinterpret_cast<const float4*>(s_w1 + 144 + quad * 4);
-        float acc[5][4];
-#pragma unroll
-        for (int p = 0; p < 5; ++p) { acc[p][0] = bq.x; acc[p][1] = bq.y; acc[p][2] = bq.z; acc[p][3] = bq.w; }
-#pragma unroll
-        for (int t = 0; t < 9; ++t) {
-            const float4 wq = *reinterpret_cast<const float4*>(s_w1 + t * PT_C1 + quad * 4);
-#pragma unroll
-            for (int p = 0; p < 5; ++p) {
-                const float xv = xw[t / 3][p + t % 3];
-                acc[p][0] = fmaf(xv, wq.x, acc[p][0]);
-                acc[p][1] = fmaf(xv, wq.y, acc[p][1]);
-                acc[p][2] = fmaf(xv, wq.z, acc[p][2]);
-                acc[p][3] = fmaf(xv, wq.w, acc[p][3]);
-            }
-        }
-        float4* plane = reinterpret_cast<float4*>(pt_smem + quad * PT_PLANE) + r * PT_HP + c0;
-#pragma unroll
-        for (int p = 0; p < 5; ++p) {
-            const int hx = x0 - 1 + c0 + p;
-            float4 o = make_float4(0.f, 0.f, 0.f, 0.f);          // conv_2's zero padding outside the image
-            if (row_in && hx >= 0 && hx < W)
-                o = make_float4(round_tf32(apply_act(acc[p][0], act1, alpha1)),
-                                round_tf32(apply_act(acc[p][1], act1, alpha1)),
-                                round_tf32(apply_act(acc[p][2], act1, alpha1)),
-                                round_tf32(apply_act(acc[p][3], act1, alpha1)));
-            plane[p] = o;
-        }
-    }
-    // generic-proxy shared-memory writes must be visible to the tensor core's async proxy
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-
-    // ---- phase 2: 18 MMAs per output row, issued by one lane of the dedicated warp 8 (its other
-    // lanes go straight to the final barrier; a lane spinning on the mbarrier in the SAME warp
-    // would starve the issuing lane)
-    if (warp == 8 && lane == 0) {
-        const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((16u >> 3) << 17) | ((128u >> 4) << 24);
-        const uint32_t sh = smem_u32(s_h), sb = smem_u32(s_b);
-#pragma unroll 1
-        for (int r = 0; r < PT_TH; ++r) {
-#pragma unroll
-            for (int t = 0; t < 9; ++t) {
-                const uint32_t pix = (uint32_t)((r + t / 3) * PT_HP + t % 3) * 16u;
-#pragma unroll
-                for (int m = 0; m < 2; ++m) {
-                    const uint64_t da = make_kmajor_nosw_desc(sh + (uint32_t)(2 * m) * PT_PLANE + pix, PT_PLANE, 128);
-                    const uint64_t db = make_kmajor_nosw_desc(sb + (uint32_t)(t * 4 + 2 * m) * 256u, 256, 128);
-                    tc_mma_tf32(tmem_base + (uint32_t)(r * 16), da, db, idesc, (t > 0 || m > 0) ? 1u : 0u);
-                }
-            }
-        }
-        tc_commit(smem_u32(bar));
-    }
-
-    // ---- phase 3: epilogue (warps 0-7), lane = pixel
-    if (warp < 8) {
-        mbar_wait(smem_u32(bar), 0);
-        tc_fence_after();
-        const int q = warp & 3, half = warp >> 2;
-        const int gx = x0 + q * 32 + lane;
-        const float bias2 = __ldg(b2);
-#pragma unroll
-        for (int rr = 0; rr < PT_TH / 2; ++rr) {
-            const int r = half * (PT_TH / 2) + rr;
-            uint32_t v;
-            asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];"
-                         : "=r"(v) : "r"(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(r * 16)) : "memory");
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-            const int gy = y0 + r;
-            if (gy < H && gx < W) yim[(int64_t)gy * W + gx] = apply_act(__uint_as_float(v) + bias2, act2, alpha2);
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
-    }
-}
-
-int conv3x3_pair_tc(const float* x, const float* w1, const float* b1, const float* w2, const float* b2, float* y,
-                    int64_t n, int64_t h, int64_t w, int c1, int act1, float alpha1, int act2, float alpha2,
-                    cudaStream_t st) {
-    if (c1 != PT_C1 || n > 65535 || ceil_div(h, PT_TH) > 65535) return UOCR_ERR_UNSUPPORTED;
-    const size_t smem = 4 * PT_PLANE + 36 * 256 + sizeof(float) * ((PT_TH + 4) * PT_XP + 160) + 16;
-    static bool configured = false;
-    if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(conv3x3_pair_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)smem);
-        if (e != cudaSuccess) { set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return UOCR_ERR_CUDA; }
-        configured = true;
-    }
-    dim3 grid((unsigned)ceil_div(w, PT_TW), (unsigned)ceil_div(h, PT_TH), (unsigned)n);
-    conv3x3_pair_tc_kernel<<<grid, PT_THREADS, smem, st>>>(x, w1, b1, w2, b2, y, (int)h, (int)w, act1, alpha1, act2, alpha2);
-    UOCR_LAUNCHED("conv3x3_pair_tc");
     return UOCR_OK;
 }
 

@@ -155,18 +155,6 @@ __device__ __forceinline__ void tc_commit_pair(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
                  ::"r"(bar), "h"((uint16_t)3) : "memory");
 }
-// ---- plain thread-block clusters (cta_group::1 MMAs): operand tiles shared by the CTAs of a cluster are fetched once
-// and delivered to every CTA named in `mask` at the same shared-memory offset (data AND the mbarrier's byte count)
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, uint16_t mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-        ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "h"(mask) : "memory");
-}
-// arrives (once) on the barrier at this shared-memory offset in every CTA of `mask` when this thread's MMAs have retired
-__device__ __forceinline__ void tc_commit_mc(uint32_t bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(bar), "h"(mask) : "memory");
-}
 __device__ __forceinline__ float round_tf32(float v) {        // the tensor core would truncate: round instead
     uint32_t u;
     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(v));

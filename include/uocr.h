@@ -229,6 +229,34 @@ int uocr_hourglass4_pack(const float* const* weights, float* packed, void* strea
 int uocr_hourglass4_fwd_packed(const float* x, const float* packed, const float* const* biases, float* y,
                                int64_t n, int64_t h, int64_t w, float alpha, int act_end, float alpha_end, void* stream);
 
+/* Ragged batches: N images of different sizes on one (N, H, W, C) canvas.  `extents` is a DEVICE table of int32
+ * (N, 2): row i = (h_i, w_i), 0 < h_i <= H, 0 < w_i <= W; image i occupies canvas[i, :h_i, :w_i, :] and everything
+ * outside that region is 0.  Every layer the networks run pads with zeros (convolutions with padding_value 0,
+ * Upsample2D, the window layer), so a valid output pixel computed on the canvas equals the pixel of the image run alone
+ * as long as every intermediate map is zero outside its own extent.  Each kernel clamps the extents to the canvas, so
+ * a bad table cannot make it write outside the canvas (it can only make the result wrong).
+ *
+ * uocr_zero_outside_hw_f32: writes 0 to every element of x outside its image's extent.  One warp per canvas row touches
+ * only the padding (16-byte stores where the alignment allows), so the cost is the padding, not the tensor.
+ * uocr_pack_hw_f32: gathers N contiguous (1, h_i, w_i, c) images into the canvas and writes its zeros, one launch.
+ * uocr_unpack_hw_f32: the inverse, scatters canvas[i, :h_i, :w_i, :] to N contiguous images.
+ * srcs / dsts: HOST arrays of N device pointers (like the weight-pointer arrays of uocr_hourglass1_fwd); the library
+ * copies them into its stream-ordered scratch, so the host array may be released when the call returns. */
+int uocr_zero_outside_hw_f32(float* x, const int32_t* extents, int64_t n, int64_t h, int64_t w, int64_t c,
+                             void* stream);
+int uocr_pack_hw_f32(const float* const* srcs, const int32_t* extents, float* canvas, int64_t n, int64_t h, int64_t w,
+                     int64_t c, void* stream);
+int uocr_unpack_hw_f32(const float* canvas, const int32_t* extents, float* const* dsts, int64_t n, int64_t h, int64_t w,
+                       int64_t c, void* stream);
+/* uocr_hourglass4_fwd_packed on a ragged batch: x (N, H, W, 1) canvas, y (N, H, W, 2) canvas, extents as above.  Each
+ * level's "inside the image" test uses the image's own extent scaled to that level, so image i's output region is
+ * bit-identical to uocr_hourglass4_fwd_packed on that image alone, and y is 0 outside it.  A CTA whose block lies
+ * wholly outside its image writes its zeros and exits.  Requires H, W, h_i and w_i to be multiples of 4 (the extents are
+ * checked on the device: a CTA of an image that breaks this writes zeros only); UOCR_ERR_UNSUPPORTED for H, W. */
+int uocr_hourglass4_fwd_packed_ragged(const float* x, const float* packed, const float* const* biases, float* y,
+                                      const int32_t* extents, int64_t n, int64_t h, int64_t w, float alpha, int act_end,
+                                      float alpha_end, void* stream);
+
 /* Backward of the same pair in TRAINING (y = conv3x3(act1(conv3x3(x, w1) + b1), w2) + b2, the final
  * activation handled by its own layer): dw1/db1/dw2/db2 (+)= parameter gradients, dx = input gradient
  * (skipped when dx == NULL), from x and dy = dL/dy only -- the c_mid-channel hidden map is recomputed

@@ -70,6 +70,7 @@ constexpr int OFF_B = OFF_R0_END;
 constexpr int OFF_BIAS = OFF_B + H4_BFLOATS * 4;
 constexpr int OFF_BAR = OFF_BIAS + 96;
 constexpr int OFF_TMEM = OFF_BAR + 64;
+constexpr int OFF_EXT = OFF_BIAS + 72;            // ragged batches: the image's extent (int2) after the 18 biases
 constexpr int H4_SMEM = OFF_TMEM + 16;
 static_assert(OFF_XO % 128 == 0 && OFF_P00 % 16 == 0 && OFF_D2 % 16 == 0 && OFF_U2 % 16 == 0 && OFF_B % 16 == 0 &&
               OFF_BAR % 8 == 0, "alignment");
@@ -81,6 +82,7 @@ struct Hourglass4Params {
     int H, W;
     float alpha;
     int act_end; float alpha_end;
+    const int32_t* ext;                           // ragged batches: (N, 2) extents (h_i, w_i) on the device
 };
 
 // ---- B operand image.  Every MMA tile is K-major [chunk c: 2][n: 16][e: 4] (k = 4 c + e); weights are (5,5,Cin,Cout).
@@ -166,12 +168,32 @@ __device__ __forceinline__ void h4_store4(uint32_t addr, const uint32_t* v, cons
 __device__ __forceinline__ void h4_zero16(uint32_t addr) {
     asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(addr), "r"(0u) : "memory");
 }
+// a ragged CTA outside its image: zeros over its 16 x 128 output block (out of line: inlined, it costs the kernel spills)
+__device__ __noinline__ void h4_zero_block(const Hourglass4Params& p, int img, int oy0, int ox0) {
+    const int gx = ox0 + (threadIdx.x & (H4_TW - 1));
+    if (gx < p.W)
+        for (int r = threadIdx.x / H4_TW; r < H4_TH && oy0 + r < p.H; r += H4_THREADS / H4_TW)
+            *reinterpret_cast<float2*>(p.y + (((int64_t)img * p.H + oy0 + r) * p.W + gx) * 2) = make_float2(0.f, 0.f);
+}
+
+// the image's extent (h, w) for the "inside the image" tests: the canvas size, or in a ragged batch the image's own
+// extent, parked in shared memory and re-read where it is used (kept in registers it pushes the kernel into spills)
+template <bool RAGGED>
+__device__ __forceinline__ int2 h4_extent(uint32_t sm, const Hourglass4Params& p) {
+    if constexpr (!RAGGED) return make_int2(p.H, p.W);
+    int2 e;
+    asm volatile("ld.shared.v2.s32 {%0, %1}, [%2];" : "=r"(e.x), "=r"(e.y) : "r"(sm + OFF_EXT));
+    return e;
+}
 __device__ __forceinline__ float4 h4_lds4(uint32_t addr) {
     float4 r;
     asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "r"(addr));
     return r;
 }
 
+// RAGGED: x and y are canvases of a ragged batch (uocr.h); every "inside the image" test uses image img's own extent
+// extent instead of the canvas size (h4_extent), while addresses keep the canvas pitch.
+template <bool RAGGED>
 __global__ void __launch_bounds__(H4_THREADS, 3) hourglass4_fwd_kernel(const Hourglass4Params p,
                                                                        const __grid_constant__ CUtensorMap map_even,
                                                                        const __grid_constant__ CUtensorMap map_odd) {
@@ -183,6 +205,17 @@ __global__ void __launch_bounds__(H4_THREADS, 3) hourglass4_fwd_kernel(const Hou
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, quarter = warp & 3;
     const int ox0 = blockIdx.x * H4_TW, oy0 = blockIdx.y * H4_TH, img = blockIdx.z;
     const int hy0 = oy0 / 2, hx0 = ox0 / 2, qy0 = oy0 / 4, qx0 = ox0 / 4;
+    if constexpr (RAGGED) {
+        int eh = min(max(__ldg(p.ext + 2 * img), 0), p.H), ew = min(max(__ldg(p.ext + 2 * img + 1), 0), p.W);
+        if ((eh | ew) & 3) eh = ew = 0;                                  // not a multiple of 4: no image, zeros only
+        if (oy0 >= eh || ox0 >= ew) {
+            // the block lies wholly outside the image: its zeros, then exit before any barrier, TMA copy or tensor
+            // memory exists (a CTA that exits with a TMA copy in flight faults, DESIGN.md §3)
+            h4_zero_block(p, img, oy0, ox0);
+            return;
+        }
+        if (tid == 0) *reinterpret_cast<int2*>(h4_smem + OFF_EXT) = make_int2(eh, ew);
+    }
 
     if (tid == 0) {
 #pragma unroll
@@ -240,14 +273,15 @@ __global__ void __launch_bounds__(H4_THREADS, 3) hourglass4_fwd_kernel(const Hou
         tc_wait_ld();
         const int m = t * 128 + quarter * 32 + lane, r = m / H4_POS, q = m - r * H4_POS;
         if (r < H4_D1H) {
-            const bool rowin = (unsigned)(hy0 - 6 + r) < (unsigned)(p.H / 2);
+            const int2 e = h4_extent<RAGGED>(sm, p);
+            const bool rowin = (unsigned)(hy0 - 6 + r) < (unsigned)(e.x / 2);
             const uint32_t plane = sm + ((r & 1) ? OFF_P10 : OFF_P00) + ((r >> 1) * H4_POS + q) * 16;
             const uint32_t pbytes = (r & 1) ? P1_BYTES : P0_BYTES;
             // position q = block columns 4 q .. 4 q + 3 = D1 columns 2 q - 1 (odd: plane 1, column q - 1) and 2 q (even:
             // plane 0, column q)
             const int col = 2 * q - 1;
-            const bool in0 = rowin && col >= 0 && (unsigned)(hx0 - 6 + col) < (unsigned)(p.W / 2);
-            const bool in1 = rowin && col + 1 < H4_D1W && (unsigned)(hx0 - 6 + col + 1) < (unsigned)(p.W / 2);
+            const bool in0 = rowin && col >= 0 && (unsigned)(hx0 - 6 + col) < (unsigned)(e.y / 2);
+            const bool in1 = rowin && col + 1 < H4_D1W && (unsigned)(hx0 - 6 + col + 1) < (unsigned)(e.y / 2);
             if (q > 0) h4_store4(plane + pbytes - 16, v, bias, p.alpha, in0);
             h4_store4(plane, v + 4, bias, p.alpha, in1);
             if (q == H4_POS - 1) h4_zero16(plane + pbytes);
@@ -288,7 +322,8 @@ __global__ void __launch_bounds__(H4_THREADS, 3) hourglass4_fwd_kernel(const Hou
         tc_wait_ld();
         const int m = t * 128 + quarter * 32 + lane, r = m / H4_POS, c = m - r * H4_POS;
         if (r < H4_D2H) {
-            const bool in = c < H4_D2W && (unsigned)(qy0 - 2 + r) < (unsigned)(p.H / 4) && (unsigned)(qx0 - 2 + c) < (unsigned)(p.W / 4);
+            const int2 e = h4_extent<RAGGED>(sm, p);
+            const bool in = c < H4_D2W && (unsigned)(qy0 - 2 + r) < (unsigned)(e.x / 4) && (unsigned)(qx0 - 2 + c) < (unsigned)(e.y / 4);
             h4_store4(sm + OFF_D2 + m * 16, v, bias, p.alpha, in);
         }
     }
@@ -317,12 +352,13 @@ __global__ void __launch_bounds__(H4_THREADS, 3) hourglass4_fwd_kernel(const Hou
         tc_wait_ld();
         const int m = t * 128 + quarter * 32 + lane, j = m / H4_POS, n = m - j * H4_POS;
         if (j < H4_U2H / 2 && n < H4_U2W / 2) {
+            const int2 e = h4_extent<RAGGED>(sm, p);
 #pragma unroll
             for (int py = 0; py < 2; ++py) {
-                const bool rowin = (unsigned)(hy0 - 2 + 2 * j + py) < (unsigned)(p.H / 2);
+                const bool rowin = (unsigned)(hy0 - 2 + 2 * j + py) < (unsigned)(e.x / 2);
 #pragma unroll
                 for (int px = 0; px < 2; ++px) {
-                    const bool in = rowin && (unsigned)(hx0 - 2 + 2 * n + px) < (unsigned)(p.W / 2);
+                    const bool in = rowin && (unsigned)(hx0 - 2 + 2 * n + px) < (unsigned)(e.y / 2);
                     h4_store4(sm + OFF_U2 + ((2 * j + py) * H4_PU2 + 2 * n + px) * 16, v + 4 * (2 * py + px), bias, p.alpha, in);
                 }
             }
@@ -353,12 +389,13 @@ __global__ void __launch_bounds__(H4_THREADS, 3) hourglass4_fwd_kernel(const Hou
         tc_wait_ld();
         const int m = t * 128 + quarter * 32 + lane, j = m / H4_PU2, n = m - j * H4_PU2;
         if (j < H4_U1H / 2 && n < H4_U1W / 2) {
+            const int2 e = h4_extent<RAGGED>(sm, p);
 #pragma unroll
             for (int py = 0; py < 2; ++py) {
-                const bool rowin = (unsigned)(oy0 - 2 + 2 * j + py) < (unsigned)p.H;
+                const bool rowin = (unsigned)(oy0 - 2 + 2 * j + py) < (unsigned)e.x;
 #pragma unroll
                 for (int px = 0; px < 2; ++px) {
-                    const bool in = rowin && (unsigned)(ox0 - 2 + 2 * n + px) < (unsigned)p.W;
+                    const bool in = rowin && (unsigned)(ox0 - 2 + 2 * n + px) < (unsigned)e.y;
                     h4_store4(sm + OFF_U1 + ((2 * j + py) * H4_PU1 + 2 * n + px) * 16, v + 4 * (2 * py + px), bias, p.alpha, in);
                 }
             }
@@ -409,6 +446,12 @@ __global__ void __launch_bounds__(H4_THREADS, 3) hourglass4_fwd_kernel(const Hou
                 o[i] = t > 0.f ? t : t * a;
             }
         }
+        if constexpr (RAGGED) {                                          // the canvas outside the extent gets zeros
+            const int2 e = h4_extent<RAGGED>(sm, p);
+#pragma unroll
+            for (int i = 0; i < 8; ++i)
+                if (gx >= e.y || oy0 + 8 * g + i >= e.x) o[2 * i] = o[2 * i + 1] = 0.f;
+        }
         if (gx < p.W) {
             float* dst = p.y + (((int64_t)img * p.H + oy0 + 8 * g) * p.W + gx) * 2;
 #pragma unroll
@@ -430,7 +473,8 @@ static int hourglass4_pack(const float* const* w, float* packed, cudaStream_t st
 }
 
 static int hourglass4_run(const float* x, const float* packed, const float* const* b, float* y, int64_t n, int64_t h,
-                          int64_t wd, float alpha, int act_end, float alpha_end, cudaStream_t st) {
+                          int64_t wd, float alpha, int act_end, float alpha_end, cudaStream_t st,
+                          const int32_t* extents = nullptr) {
     if (h % 4 || wd % 4 || n > 65535 || alpha < 0.f || alpha > 1.f) return UOCR_ERR_UNSUPPORTED;
     if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(packed)) & 15)
         return UOCR_ERR_UNSUPPORTED;
@@ -443,18 +487,25 @@ static int hourglass4_run(const float* x, const float* packed, const float* cons
     if (rc != UOCR_OK) return rc;
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(hourglass4_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, H4_SMEM);
-        if (e != cudaSuccess) { set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return UOCR_ERR_CUDA; }
+        for (const void* kernel : {(const void*)hourglass4_fwd_kernel<false>, (const void*)hourglass4_fwd_kernel<true>}) {
+            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, H4_SMEM);
+            if (e != cudaSuccess) { set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return UOCR_ERR_CUDA; }
+        }
         configured = true;
     }
     Hourglass4Params p{};
     p.y = y; p.bimg = packed;
     for (int l = 0; l < 5; ++l) p.b[l] = b[l];
-    p.H = (int)h; p.W = (int)wd; p.alpha = alpha; p.act_end = act_end; p.alpha_end = alpha_end;
+    p.H = (int)h; p.W = (int)wd; p.alpha = alpha; p.act_end = act_end; p.alpha_end = alpha_end; p.ext = extents;
     dim3 grid((unsigned)ceil_div(wd, H4_TW), (unsigned)ceil_div(h, H4_TH), (unsigned)n);
     if (grid.y > 65535) return UOCR_ERR_UNSUPPORTED;
-    hourglass4_fwd_kernel<<<grid, H4_THREADS, H4_SMEM, st>>>(p, map_even, map_odd);
-    UOCR_LAUNCHED("hourglass4_fwd");
+    if (extents) {
+        hourglass4_fwd_kernel<true><<<grid, H4_THREADS, H4_SMEM, st>>>(p, map_even, map_odd);
+        UOCR_LAUNCHED("hourglass4_fwd_ragged");
+    } else {
+        hourglass4_fwd_kernel<false><<<grid, H4_THREADS, H4_SMEM, st>>>(p, map_even, map_odd);
+        UOCR_LAUNCHED("hourglass4_fwd");
+    }
     return UOCR_OK;
 }
 
@@ -491,6 +542,18 @@ extern "C" int uocr_hourglass4_fwd_packed(const float* x, const float* packed, c
     if (rc != UOCR_OK) return rc;
     rc = hourglass4_run(x, packed, biases, y, n, h, w, alpha, act_end, alpha_end, as_stream(stream));
     if (rc == UOCR_ERR_UNSUPPORTED) set_error("hourglass4_fwd: unsupported geometry (H, W must be multiples of 4)");
+    return rc;
+}
+
+extern "C" int uocr_hourglass4_fwd_packed_ragged(const float* x, const float* packed, const float* const* biases, float* y,
+                                                 const int32_t* extents, int64_t n, int64_t h, int64_t w, float alpha,
+                                                 int act_end, float alpha_end, void* stream) {
+    UOCR_REQUIRE(packed && extents, "NULL pointer");
+    int rc = hourglass4_check(x, y, biases, n, h, w, act_end);
+    if (rc != UOCR_OK) return rc;
+    rc = hourglass4_run(x, packed, biases, y, n, h, w, alpha, act_end, alpha_end, as_stream(stream), extents);
+    if (rc == UOCR_ERR_UNSUPPORTED)
+        set_error("hourglass4_fwd_packed_ragged: unsupported geometry (H, W and every extent must be multiples of 4)");
     return rc;
 }
 

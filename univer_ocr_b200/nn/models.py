@@ -17,11 +17,13 @@ replayed; no layer call synchronises the device, and loss values stay on the dev
 """
 import ctypes
 
+import numpy as np
+
 from .._lib import ACT_LEAKY, ACT_NONE, ACT_SIGMOID, MATH_TF32, lib
 from .gpu import CP, DeviceArray, LazyScalar, as_device, stream
 from .help_func import make_list_if_not
 from .layers import (BaseLayer, Conv2DToBatchedFixedWidthed, Convolutional2D, Flatten, FromOutput, FullyConnected,
-                     LeakyRelu, Sigmoid, Upsample2D, _kmajor_copy)
+                     LeakyRelu, Relu, Sigmoid, Upsample2D, _kmajor_copy)
 from .losses import SoftmaxCrossEntropy
 from .progress_tracker import track_method
 
@@ -224,7 +226,9 @@ class Model(BaseModel):
             return None
         return dst
 
-    def _make_plan(self, training):
+    def _make_plan(self, training, ragged=False):
+        """`ragged`: the inference plan of `predict_ragged`, without the Monochrome pair kernel, whose C-channel
+        intermediate stays on chip where it cannot be zeroed outside each image's extent."""
         plan, taken = [], set()
         for name in self._order:
             if name in taken:
@@ -251,7 +255,7 @@ class Model(BaseModel):
                     if act is None or (training and act[0] != ACT_LEAKY):
                         act_name = None
                     pair = None
-                    if (ups is None and act_name is not None and type(conv) is Convolutional2D
+                    if (ups is None and act_name is not None and type(conv) is Convolutional2D and not ragged
                             and self._pair_head(conv)
                             and (not training or act[0] == ACT_LEAKY)):
                         c2_name = self._sole_consumer(act_name)
@@ -312,7 +316,6 @@ class Model(BaseModel):
         inputs = make_list_if_not(inputs)
         if not self.is_initialized:
             self.initialize_from_X(inputs)
-        outputs = {}
         if not training and self._fusion_planned and self.infer_fusion is not None:
             fused = self.infer_fusion(self, inputs)
             if fused is not None:
@@ -320,10 +323,18 @@ class Model(BaseModel):
                                        **{k: fused[k] for k in range(self.outputs_count)}}
                 return fused
 
+        outputs = self._run_steps(self._plan_train if training else self._plan_infer, inputs, training, clear_grads)
+        self.layers_outputs = outputs
+        return [outputs[k] for k in range(self.outputs_count)]
+
+    def _run_steps(self, plan, inputs, training, clear_grads, after_step=None):
+        """Runs `plan` on `inputs` -> {layer name / output index: value}; `after_step(step, outputs)` after each step."""
+        outputs = {}
+
         def value_of(src):
             return inputs[src] if isinstance(src, int) else outputs[src]
 
-        for step in (self._plan_train if training else self._plan_infer):
+        for step in plan:
             kind = step[0]
             if kind == 'layer':
                 name = step[1]
@@ -344,10 +355,11 @@ class Model(BaseModel):
                         if member is not None:
                             self.layers[member].clear_grads()
                 self._run_pair(step, value_of, outputs, training)
+            if after_step is not None:
+                after_step(step, outputs)
         for key in self._output_keys():
             outputs[key] = value_of(self.relations[key][0])
-        self.layers_outputs = outputs
-        return [outputs[k] for k in range(self.outputs_count)]
+        return outputs
 
     def _run_fused_conv(self, step, value_of, outputs, training, clear_grads=True):
         _, ups_name, conv_name, act_name = step
@@ -609,6 +621,122 @@ class Model(BaseModel):
     def predict(self, X):
         return self.forward(X, training=False)
 
+    # ---- ragged batches -----------------------------------------------------------
+    # Layers whose zero padding makes a canvas of zero-padded images exact (DESIGN.md §3).  Relu is listed apart from
+    # LeakyRelu because the check is by exact type.
+    RAGGED_LAYERS = (Convolutional2D, Upsample2D, LeakyRelu, Relu, Sigmoid, Conv2DToBatchedFixedWidthed, Flatten,
+                     FullyConnected)
+    _plan_ragged = None
+
+    def ragged_analysis(self, canvas_shape, extents):
+        """Host-side analysis of a ragged batch: a canvas (N, H, W, C) holding image i in [i, :h_i, :w_i, :] with
+        (h_i, w_i) = extents[i].  Raises ValueError for extents outside the canvas and for layers a ragged batch cannot
+        run through.  -> (extents as int64 (N, 2), {layer name: ('hw', (N, 2) per-image (h, w) of its output, the canvas
+        output's (H, W)) or ('rows', (N, 2) [first, end) row range of each image, None)}).  The per-image shapes are the model's own shape analysis
+        of (1, h_i, w_i, C), one analysis per distinct extent.  After a Conv2DToBatchedFixedWidthed the batch axis holds
+        one row per window: image i owns rows [i * W, i * W + w_i) of it, W and w_i the canvas and image widths there."""
+        assert self.is_initialized, 'The model must be initialized before calling this method'
+        for name, layer in self.layers.items():
+            if type(layer) not in self.RAGGED_LAYERS:
+                raise ValueError(f'{name}: {type(layer).__name__} is not supported on ragged batches')
+            if type(layer) is Convolutional2D and layer.padding_value != 0:
+                raise ValueError(f'{name}: padding_value {layer.padding_value} != 0 is not supported on ragged batches')
+        if self.inputs_count != 1:
+            raise ValueError(f'ragged batches need a model with one input, this one has {self.inputs_count}')
+        shape = tuple(int(v) for v in canvas_shape)
+        if len(shape) != 4:
+            raise ValueError(f'a ragged canvas is (N, H, W, C), got shape {shape}')
+        n, H, W, C = shape
+        ext = np.asarray(extents)
+        if ext.shape != (n, 2) or not (ext.dtype.kind in 'iu' or ext.size == 0):
+            raise ValueError(f'extents must be an integer ({n}, 2) array, got {ext.dtype} {ext.shape}')
+        ext = ext.astype(np.int64)
+        bad = np.flatnonzero((ext[:, 0] < 1) | (ext[:, 0] > H) | (ext[:, 1] < 1) | (ext[:, 1] > W))
+        if bad.size:
+            i = int(bad[0])
+            raise ValueError(f'extent {i} = {tuple(int(v) for v in ext[i])} is outside the {H} x {W} canvas')
+        canvas_shapes = self.get_all_output_shapes([shape])[1]
+        per_extent = {}
+        for h, w in sorted(set(map(tuple, ext.tolist()))):
+            try:
+                per_extent[h, w] = self.get_all_output_shapes([(1, h, w, C)])[1]
+            except AssertionError as e:
+                raise ValueError(f'extent {h} x {w}: {e}') from None
+        keys = [tuple(e) for e in ext.tolist()]
+        modes = {}
+
+        def mode_of(src):
+            return ('hw', ext, (H, W)) if isinstance(src, int) else modes[src]
+
+        def canvas_of(src):
+            return shape if isinstance(src, int) else canvas_shapes[src][0]
+
+        for name in self._order:
+            layer, srcs = self.layers[name], self.relations[name]
+            kinds = {mode_of(src)[0] for src in srcs}
+            if kinds == {'rows'}:
+                modes[name] = mode_of(srcs[0])
+            elif kinds != {'hw'}:
+                raise ValueError(f'{name}: mixes image maps and window rows')
+            elif type(layer) is Conv2DToBatchedFixedWidthed:
+                (_, hc, wc, _), table = canvas_of(srcs[0]), mode_of(srcs[0])[1]
+                if (table[:, 0] != hc).any():
+                    raise ValueError(f'{name}: windows of images shorter than the canvas would carry its padding')
+                first = np.arange(n, dtype=np.int64) * wc
+                modes[name] = ('rows', np.stack([first, first + table[:, 1]], axis=1), None)
+            elif type(layer) in (Flatten, FullyConnected):
+                raise ValueError(f'{name}: {type(layer).__name__} of a ragged image map would mix in its padding')
+            else:
+                table = np.array([per_extent[k][name][0][1:3] for k in keys], dtype=np.int64).reshape(n, 2)
+                _, hc, wc, _ = canvas_of(name)
+                if (table[:, 0] > hc).any() or (table[:, 1] > wc).any():
+                    raise ValueError(f'{name}: an image output is larger than the canvas output {hc} x {wc}')
+                modes[name] = ('hw', table, (hc, wc))
+        return ext, modes
+
+    def predict_ragged(self, canvas, extents):
+        """Inference on a ragged batch: `canvas` (N, H, W, C) device (or host) array, zero outside each image, image i
+        in canvas[i, :h_i, :w_i, :]; `extents` host (N, 2) integers (h_i, w_i).  -> (outputs, output extents): one output
+        canvas per model output and, per output, an (N, 2) int64 array -- (h_i, w_i) of image i's region for an image
+        map, [first, end) of image i's rows after a Conv2DToBatchedFixedWidthed (see `ragged_analysis`).  Image i's
+        region equals `predict` on that image alone, up to the rounding of shape-dependent kernel choices, and image maps
+        are 0 outside it.  Every step that outputs an image map is followed by uocr_zero_outside_hw_f32 where some extent
+        is smaller than the canvas; fused steps that keep a spatial map on chip step aside for their materialising
+        equivalents (the Paragraph one-kernel, the Monochrome pair kernel), the Line one-kernel runs its ragged variant
+        when every extent is a multiple of 4.  Extents and layers are checked before anything is launched."""
+        ext, modes = self.ragged_analysis(canvas.shape, extents)
+        out_names = [self.relations[k][0] for k in range(self.outputs_count)]
+
+        def out_table(src):
+            return ext.copy() if isinstance(src, int) else modes[src][1].copy()
+
+        # every extent table a kernel reads, uploaded in one copy: the input's, then one per masked output
+        tables, offsets = [ext], {}
+        for name in self._order:
+            kind, table, canvas_hw = modes[name]
+            if kind == 'hw' and ((table[:, 0] < canvas_hw[0]) | (table[:, 1] < canvas_hw[1])).any():
+                offsets[name] = sum(t.size for t in tables)
+                tables.append(table)
+        dev = DeviceArray.from_host(np.concatenate(tables).astype(np.int32), np.int32)
+        X = as_device(canvas)
+        if self._fusion_planned and isinstance(self.infer_fusion, HourglassFusion):
+            fused = self.infer_fusion(self, [X], ext, dev.ptr)
+            if fused is not None:
+                self.layers_outputs = {**{name: None for name in self.layers}, 0: fused[0]}
+                return fused, [out_table(out_names[0])]
+        if self._plan_ragged is None:
+            self._plan_ragged = self._make_plan(training=False, ragged=True) if self._fusion_planned else self._plan_infer
+
+        def mask(step, outputs):
+            name = [m for m in step[1:] if m is not None][-1]
+            if name in offsets:
+                y = outputs[name]
+                lib.uocr_zero_outside_hw_f32(y.ptr, dev.ptr + 4 * offsets[name], *y.shape, stream())
+
+        outputs = self._run_steps(self._plan_ragged, [X], False, True, after_step=mask)
+        self.layers_outputs = outputs
+        return [outputs[k] for k in range(self.outputs_count)], [out_table(src) for src in out_names]
+
     def update_grads(self):
         if not self.trainable:
             return
@@ -857,11 +985,11 @@ class HourglassFusion:
             return None
         return out
 
-    def __call__(self, model, inputs):
+    def _applies(self, model, X):
+        """(blocks, inner activations, end activation, four-channel) if the kernel takes `X`, else None."""
         blocks = self._blocks(model)
         if blocks is None:
             return None
-        X = as_device(inputs[0])
         if len(X.shape) != 4 or X.shape[3] != 1 or X.shape[1] % 4 or X.shape[2] % 4 or X.shape[0] > 65535:
             return None
         inner = [_act_code(act) for _, act in blocks[:4]]
@@ -872,6 +1000,29 @@ class HourglassFusion:
         four = blocks[1][0].in_channels == 4
         if four and CP.math_mode != MATH_TF32:             # the four-channel kernel is tensor-core (TF32) only
             return None
+        return blocks, inner, end, four
+
+    def _packed_image(self, blocks, wp):
+        key = (CP.weights_generation, tuple(conv.w.value.ptr for conv, _ in blocks))
+        if self._packed is None or self._packed[0] != key:         # tensor-core operand image of the five weight tensors
+            count = ctypes.c_int64()
+            lib.uocr_hourglass4_packed_floats(ctypes.byref(count))
+            packed = DeviceArray((count.value,))
+            lib.uocr_hourglass4_pack(wp, packed.ptr, stream())
+            self._packed = (key, packed)
+        return self._packed[1]
+
+    def __call__(self, model, inputs, extents=None, extents_ptr=None):
+        """`extents` (host (N, 2)) / `extents_ptr` (the same table on the device): a ragged batch (Model.predict_ragged),
+        run by the four-channel kernel's ragged variant when every extent is a multiple of 4; None (-> the layer plan)
+        for every other ragged case, since the one-channel kernel keeps its maps on chip where they cannot be masked."""
+        X = as_device(inputs[0])
+        found = self._applies(model, X)
+        if found is None:
+            return None
+        blocks, inner, end, four = found
+        if extents is not None and (not four or (np.asarray(extents) % 4).any()):
+            return None
         n, h, w, _ = X.shape
         ptrs = ctypes.c_void_p * 5
         wp = ptrs(*[conv.w.value.ptr for conv, _ in blocks])
@@ -879,16 +1030,12 @@ class HourglassFusion:
         last = blocks[4][1]
         last.progress_tracker.start_tracking(last.name, 'forward')
         y = DeviceArray((n, h, w, blocks[4][0].out_channels))
-        if four:
-            key = (CP.weights_generation, tuple(conv.w.value.ptr for conv, _ in blocks))
-            if self._packed is None or self._packed[0] != key:         # tensor-core operand image of the five weight tensors
-                count = ctypes.c_int64()
-                lib.uocr_hourglass4_packed_floats(ctypes.byref(count))
-                packed = DeviceArray((count.value,))
-                lib.uocr_hourglass4_pack(wp, packed.ptr, stream())
-                self._packed = (key, packed)
-            lib.uocr_hourglass4_fwd_packed(X.ptr, self._packed[1].ptr, bp, y.ptr, n, h, w, inner[0][1], end[0], end[1],
-                                           stream())
+        if extents is not None:
+            lib.uocr_hourglass4_fwd_packed_ragged(X.ptr, self._packed_image(blocks, wp).ptr, bp, y.ptr, extents_ptr, n, h,
+                                                  w, inner[0][1], end[0], end[1], stream())
+        elif four:
+            lib.uocr_hourglass4_fwd_packed(X.ptr, self._packed_image(blocks, wp).ptr, bp, y.ptr, n, h, w, inner[0][1],
+                                           end[0], end[1], stream())
         else:
             lib.uocr_hourglass1_fwd_mode(X.ptr, wp, bp, y.ptr, n, h, w, inner[0][1], end[0], end[1], CP.math_mode, stream())
         last.progress_tracker.stop_tracking(last.name, 'forward')

@@ -228,19 +228,36 @@ class CropAndRotateParagraphs:
     def __call__(self, masks, images):
         images = [_device(image) for image in images]
         labels, objects = label_objects(masks)
-        # per paragraph: the object's mask and the masked maps, cut to its box (CropAndRotateSingleParagraph._run, :300-309)
+        cut = self.cut(labels, objects, images)
+        self.angles = self.search_angles([cut])[0]
+        return self.straighten(cut, self.angles, len(images))
+
+    # The three phases of a call, also run by predict.TextPipeline.batch over the paragraphs of many pages at once.
+    @staticmethod
+    def cut(labels, objects, images):
+        """Per paragraph of a (1, H, W, 1) label map and its `glue.label_stats` objects: the object's mask and the masked
+        maps, cut to its box (CropAndRotateSingleParagraph._run, :300-309)."""
         cut = []
         for paragraph_id, obj in enumerate(objects):
             region_y, region_x = obj['slices']
             mask = crop_label_mask(labels, paragraph_id + 1, region_y, region_x)
             cut.append((mask, [crop(image, region_y, region_x, labels, paragraph_id + 1) for image in images]))
-        # ._func (:312-343): the angle (all paragraphs searched in lockstep), the rotated mask's box, the rotated maps cut to it
-        if self.find_rotation:
-            self.angles = find_rotation_angles([mask for mask, _ in cut], self.EPS)
-        else:
-            self.angles = [None] * len(cut)
-        result = [[None for _ in objects] for _ in images]
-        for paragraph_id, ((mask, arrays), angle) in enumerate(zip(cut, self.angles)):
+        return cut
+
+    def search_angles(self, cuts):
+        """._func (:312-343), first part: the angle of every paragraph of every `cut` result, all searched in lockstep."""
+        masks = [mask for cut in cuts for mask, _ in cut]
+        angles = find_rotation_angles(masks, self.EPS) if self.find_rotation else [None] * len(masks)
+        out, pos = [], 0
+        for cut in cuts:
+            out.append(angles[pos:pos + len(cut)])
+            pos += len(cut)
+        return out
+
+    def straighten(self, cut, angles, image_count):
+        """._func, second part: the rotated mask's box, the rotated maps cut to it -> result[image_id][paragraph_id]."""
+        result = [[None for _ in cut] for _ in range(image_count)]
+        for paragraph_id, ((mask, arrays), angle) in enumerate(zip(cut, angles)):
             out_y, out_x = mask_bbox(rotate_array(mask, angle, good_rotation=False))
             for image_id, arr in enumerate(arrays):
                 res = crop(rotate_array(arr, angle), out_y, out_x)

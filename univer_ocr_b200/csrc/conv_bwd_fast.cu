@@ -727,19 +727,20 @@ int conv_wgrad_fast(const ConvGeom& g, int math_mode, const float* x, const floa
     int nblk, chunks, nout;
     small_wgrad_dims(g, p, &nblk, &chunks, &nout);
     if (chunks > 65535) return UOCR_ERR_UNSUPPORTED;
+    const bool roll = g.kw == 5 && g.sh == 1 && g.cin == 1 && g.cout == 1 && g.w % 2 == 0 && g.wo % 4 == 0 &&
+                      g.ph == 2 && g.pw == 2;
+    if (g.ups != 1 && !roll) return UOCR_ERR_UNSUPPORTED;      // only the roll kernel reads an upsampled input
     int rc = UOCR_ERR_UNSUPPORTED;
     const bool k33 = g.kh == 3;
     if (k33 && g.cin == 1) rc = launch_small_wgrad<3, 3, 1, 1, 1, 1, 4, 4, 16>(g, x, dy, ws, nblk, chunks, st);
     else if (k33 && g.cin == 16) rc = launch_small_wgrad<3, 3, 1, 1, 16, 4, 1, 4, 16>(g, x, dy, ws, nblk, chunks, st);
     else if (k33 && g.cin == 4) rc = launch_small_wgrad<3, 3, 1, 1, 4, 4, 1, 4, 16>(g, x, dy, ws, nblk, chunks, st);
-    else if (g.kw == 5 && g.sh == 1 && g.cin == 1 && g.cout == 1 && g.w % 2 == 0 && g.wo % 4 == 0 && g.ph == 2 &&
-             g.pw == 2) {
+    else if (roll) {
         if (g.ups == 2) conv55_c1_wgrad_roll_kernel<16, true><<<dim3(nblk, chunks), 256, 0, st>>>(g, x, dy, ws, nblk);
         else conv55_c1_wgrad_roll_kernel<16, false><<<dim3(nblk, chunks), 256, 0, st>>>(g, x, dy, ws, nblk);   // plan: px 8, r 16
         UOCR_LAUNCHED("conv55_c1_wgrad_roll");
         rc = UOCR_OK;
     }
-    else if (g.ups != 1) return UOCR_ERR_UNSUPPORTED;      // only the kernel above reads an upsampled input
     else if (g.kw == 5 && g.sh == 1 && g.cin == 1) rc = launch_small_wgrad<5, 5, 1, 1, 1, 1, 1, 8, 16>(g, x, dy, ws, nblk, chunks, st);
     else if (g.kw == 5 && g.sh == 2 && g.cin == 1 && p.cot == 1) rc = launch_small_wgrad<5, 5, 2, 2, 1, 1, 1, 4, 4>(g, x, dy, ws, nblk, chunks, st);
     else if (g.kw == 5 && g.sh == 2 && g.cin == 1 && p.cot == 2) rc = launch_small_wgrad<5, 5, 2, 2, 1, 1, 2, 4, 2>(g, x, dy, ws, nblk, chunks, st);

@@ -384,6 +384,25 @@ int uocr_seg_grad(const float* gt, const float* x_pre, float* out, int64_t n, in
  * 0 * log 0 -> NaN as in the reference.   replaces: losses.py:60-73 */
 int uocr_softmax_ce(const float* logits, const float* gt, float* grad, float* loss, int64_t batch,
                     int64_t classes, float* workspace /* batch floats */, void* stream);
+/* Losses of a ragged batch (the canvas layout of uocr_zero_outside_hw_f32; extents / ranges are int32 device tables,
+ * clamped to the canvas, so a bad table makes results wrong but never makes a kernel access memory outside its buffers).
+ *
+ * uocr_seg_loss_ragged: uocr_seg_loss on (N, H, W, C) canvases where only image n's h_n x w_n region counts: the
+ * per-(n, c) sums read nothing outside it, the finalize step is uocr_seg_loss's (loss = the sum of the per-image
+ * losses), and grad, when non-NULL, is a * gt + b inside each extent and 0 outside it.  Same workspace as uocr_seg_loss.
+ * uocr_seg_grad_ragged: uocr_seg_grad of a ragged batch: the gradient (times the Sigmoid derivative when x_pre != NULL)
+ * inside each extent, 0 outside it, written in one pass over the canvas.
+ * uocr_softmax_ce_rows: uocr_softmax_ce over the rows of the n_images [first, end) ranges of a windowed ragged batch
+ * (ranges (n_images, 2), sorted by first; row r belongs to the last range with first <= r if r < its end).  loss =
+ * -sum over those rows of sum(gt * log p) / denom, grad = (p - gt) / denom there and 0 in every other row, which adds
+ * nothing to the loss.  denom > 0 is the caller's: the number of valid rows, or their count over all data-parallel
+ * ranks.  0 * log 0 -> NaN as in uocr_softmax_ce.  workspace: batch floats. */
+int uocr_seg_loss_ragged(int kind, const float* pred, const float* gt, float* grad, float* loss, const int32_t* extents,
+                         int64_t n, int64_t h, int64_t w, int64_t c, void* workspace, void* stream);
+int uocr_seg_grad_ragged(const float* gt, const float* x_pre, float* out, const int32_t* extents, int64_t n, int64_t h,
+                         int64_t w, int64_t c, const void* workspace, void* stream);
+int uocr_softmax_ce_rows(const float* logits, const float* gt, float* grad, float* loss, const int32_t* ranges,
+                         int64_t n_images, int64_t batch, int64_t classes, float denom, float* workspace, void* stream);
 /* replaces: losses.py:45-57 */
 int uocr_sigmoid_ce(const float* logits, const float* gt, float* grad, float* loss, int64_t batch,
                     int64_t classes, void* stream);

@@ -104,6 +104,13 @@ __device__ __forceinline__ T block_sum(T v, T* smem /* >= 8 elements */) {
     return r;
 }
 
+// ragged batches (ragged.cu, loss_opt.cu): image i's extent (h_i, w_i) from the device table, clamped to the canvas
+__device__ __forceinline__ void ragged_extent(const int32_t* __restrict__ ext, int64_t i, int64_t h, int64_t w,
+                                              int64_t& hi, int64_t& wi) {
+    hi = min((int64_t)max(__ldg(ext + 2 * i), 0), h);
+    wi = min((int64_t)max(__ldg(ext + 2 * i + 1), 0), w);
+}
+
 // epilogue flavour for the convolution kernels: ex2.approx + fast reciprocal (|rel err| ~ 1e-6 on
 // the sigmoid, far inside the 1e-4 conv tolerance) -- the IEEE expf + divide sequence costs ~25
 // instructions per output, which made the Cin = 1 stencils issue-bound (ncu: issue slots 80 % busy)

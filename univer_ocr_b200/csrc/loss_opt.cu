@@ -100,6 +100,70 @@ __global__ void __launch_bounds__(kThreads) seg_finalize_kernel(int kind, const 
     if (threadIdx.x == 0) loss[0] = (float)acc;
 }
 
+// pass 1 of a ragged batch: the same sums over image n's h_n x w_n region of the (N, H, W, C) canvas only.
+// grid = (chunks, N): the chunks split the region's rows, one warp per row; a row is w_n * c contiguous floats, read
+// with 16-byte loads where the alignment allows (c == 1).
+__global__ void __launch_bounds__(kThreads) seg_sums_ragged_kernel(const float* __restrict__ pred,
+                                                                   const float* __restrict__ gt,
+                                                                   const int32_t* __restrict__ ext,
+                                                                   double* __restrict__ sums, int64_t h, int64_t w,
+                                                                   int c, int64_t nc) {
+    __shared__ double red[8];
+    const int n = blockIdx.y;
+    const int lane = threadIdx.x & 31;
+    int64_t hn, wn;
+    ragged_extent(ext, n, h, w, hn, wn);
+    const int64_t per = (hn + gridDim.x - 1) / gridDim.x;
+    const int64_t y0 = (int64_t)blockIdx.x * per, y1 = min(hn, y0 + per);
+    const int64_t len = wn * c, stride = w * c;
+    const bool al = ((reinterpret_cast<uintptr_t>(pred) ^ reinterpret_cast<uintptr_t>(gt)) & 15) == 0;
+    for (int ch = 0; ch < c; ++ch) {
+        float spg = 0.f, sp = 0.f, sg = 0.f;
+        auto add = [&](float a, float b) { spg = fmaf(a, b, spg); sp += a; sg += b; };
+        for (int64_t y = y0 + (threadIdx.x >> 5); y < y1; y += kThreads / 32) {
+            const float* p = pred + ((int64_t)n * h + y) * stride;
+            const float* g = gt + ((int64_t)n * h + y) * stride;
+            if (c == 1) {
+                // scalar head up to a 16-byte boundary of p (and g: same offset), float4 body, scalar tail
+                const int64_t head = al ? min(len, (int64_t)((4 - ((reinterpret_cast<uintptr_t>(p) >> 2) & 3)) & 3))
+                                        : len;
+                for (int64_t j = lane; j < head; j += 32) add(p[j], g[j]);
+                const int64_t quads = (len - head) >> 2;
+                const float4* p4 = reinterpret_cast<const float4*>(p + head);
+                const float4* g4 = reinterpret_cast<const float4*>(g + head);
+                for (int64_t q = lane; q < quads; q += 32) {
+                    const float4 a = p4[q], b = g4[q];
+                    spg = fmaf(a.x, b.x, spg); spg = fmaf(a.y, b.y, spg);
+                    spg = fmaf(a.z, b.z, spg); spg = fmaf(a.w, b.w, spg);
+                    sp += (a.x + a.y) + (a.z + a.w);
+                    sg += (b.x + b.y) + (b.z + b.w);
+                }
+                for (int64_t j = head + 4 * quads + lane; j < len; j += 32) add(p[j], g[j]);
+            } else {
+                for (int64_t x = lane; x < wn; x += 32) add(p[x * c + ch], g[x * c + ch]);
+            }
+        }
+        const double r0 = block_sum((double)spg, red);
+        const double r1 = block_sum((double)sp, red);
+        const double r2 = block_sum((double)sg, red);
+        if (threadIdx.x == 0) {
+            atomicAdd(&sums[0 * nc + n * c + ch], r0);
+            atomicAdd(&sums[1 * nc + n * c + ch], r1);
+            atomicAdd(&sums[2 * nc + n * c + ch], r2);
+        }
+    }
+}
+
+// one gradient element: a * gt + b, with SIG times the Sigmoid derivative e / (e + 1)^2, e = exp(-x)
+template <bool SIG>
+__device__ __forceinline__ float seg_grad_value(float a, float b, float gv, float xv) {
+    const float gr = fmaf(a, gv, b);
+    if (!SIG) return gr;
+    const float e = expf(-xv);                               // same expression as SigmoidBwd (elementwise.cu)
+    const float d = e + 1.f;
+    return gr * e / (d * d);
+}
+
 // pass 2: grad = a[n,c] * gt + b[n,c]  (SIG: times the Sigmoid derivative e / (e + 1)^2, e = exp(-x), of the
 // pre-activation x the prediction came from -- loss gradient and Sigmoid backward in one pass).  grid = (chunks, N)
 template <bool SIG>
@@ -113,13 +177,7 @@ __global__ void __launch_bounds__(kThreads) seg_grad_kernel(const float* __restr
     const float* xp = SIG ? xpre + (int64_t)n * len : nullptr;
     float* o = grad + (int64_t)n * len;
     const float* cf = coef + (int64_t)n * c * 2;
-    auto one = [&](float a, float b, float gv, float xv) {
-        const float gr = fmaf(a, gv, b);
-        if (!SIG) return gr;
-        const float e = expf(-xv);                           // same expression as SigmoidBwd (elementwise.cu)
-        const float d = e + 1.f;
-        return gr * e / (d * d);
-    };
+    auto one = [&](float a, float b, float gv, float xv) { return seg_grad_value<SIG>(a, b, gv, xv); };
     const bool al = ((reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(o) |
                       (SIG ? reinterpret_cast<uintptr_t>(xp) : 0)) & 15) == 0;
     if (c == 1 && al) {
@@ -146,10 +204,84 @@ __global__ void __launch_bounds__(kThreads) seg_grad_kernel(const float* __restr
     }
 }
 
+// pass 2 of a ragged batch: one warp per canvas row writes the whole row -- the gradient over image i's w_i * c floats
+// when the row is inside its extent, 0 everywhere else -- and reads gt / x_pre inside the extent only.  16-byte stores
+// (and loads) where the alignment allows.
+template <bool SIG>
+__global__ void __launch_bounds__(kThreads) seg_grad_ragged_kernel(const float* __restrict__ gt,
+                                                                   const float* __restrict__ coef,
+                                                                   const float* __restrict__ xpre,
+                                                                   float* __restrict__ grad,
+                                                                   const int32_t* __restrict__ ext, int64_t n,
+                                                                   int64_t h, int64_t w, int c) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warps = (int64_t)gridDim.x * (kThreads / 32);
+    const bool al = ((reinterpret_cast<uintptr_t>(grad) ^ reinterpret_cast<uintptr_t>(gt)) & 15) == 0 &&
+                    (!SIG || ((reinterpret_cast<uintptr_t>(grad) ^ reinterpret_cast<uintptr_t>(xpre)) & 15) == 0);
+    const int64_t end = w * c;
+    for (int64_t row = (int64_t)blockIdx.x * (kThreads / 32) + (threadIdx.x >> 5); row < n * h; row += warps) {
+        const int64_t i = row / h, y = row - i * h;
+        int64_t hi, wi;
+        ragged_extent(ext, i, h, w, hi, wi);
+        const int64_t len = (y < hi ? wi : 0) * c;
+        const float* g = gt + row * end;
+        const float* xp = SIG ? xpre + row * end : nullptr;
+        float* o = grad + row * end;
+        const float* cf = coef + i * c * 2;
+        auto val = [&](int64_t j, float gv, float xv) {
+            const int ch = c == 1 ? 0 : (int)(j % c);
+            return seg_grad_value<SIG>(cf[2 * ch], cf[2 * ch + 1], gv, xv);
+        };
+        auto scalar = [&](int64_t j) { return j < len ? val(j, g[j], SIG ? xp[j] : 0.f) : 0.f; };
+        const int64_t head = al ? min(end, (int64_t)((4 - ((reinterpret_cast<uintptr_t>(o) >> 2) & 3)) & 3)) : end;
+        for (int64_t j = lane; j < head; j += 32) o[j] = scalar(j);
+        const int64_t quads = (end - head) >> 2;
+        for (int64_t q = lane; q < quads; q += 32) {
+            const int64_t j = head + 4 * q;
+            float4 r = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (j + 4 <= len) {
+                const float4 gv = *reinterpret_cast<const float4*>(g + j);
+                const float4 xv = SIG ? *reinterpret_cast<const float4*>(xp + j) : make_float4(0.f, 0.f, 0.f, 0.f);
+                r = make_float4(val(j, gv.x, xv.x), val(j + 1, gv.y, xv.y), val(j + 2, gv.z, xv.z),
+                                val(j + 3, gv.w, xv.w));
+            } else if (j < len) {
+                r = make_float4(scalar(j), scalar(j + 1), scalar(j + 2), scalar(j + 3));
+            }
+            *reinterpret_cast<float4*>(o + j) = r;
+        }
+        for (int64_t j = head + 4 * quads + lane; j < end; j += 32) o[j] = scalar(j);
+    }
+}
+
 // ---------------------------------------------------------------- softmax cross-entropy
 // one warp per row.  log p is evaluated as (x - max) - log(sum) (more accurate in FP32 than
 // log(e / s)); p underflows to exactly 0 in the reference's float64 when x - max < -745.13, and
 // there log p = -inf, so 0 * log 0 = NaN and 1 * log 0 = -inf are reproduced (losses.py:71).
+// one row, one warp: row_loss[r] = sum(gt * log p), grad = (p - gt) * inv
+__device__ __forceinline__ void softmax_ce_row(const float* __restrict__ logits, const float* __restrict__ gt,
+                                               float* __restrict__ grad, float* __restrict__ row_loss, int64_t r,
+                                               int classes, float inv, int lane) {
+    const float* x = logits + r * classes;
+    const float* g = gt + r * classes;
+    float m = -INFINITY;
+    for (int j = lane; j < classes; j += 32) m = fmaxf(m, x[j]);
+    m = warp_max(m);
+    float s = 0.f;
+    for (int j = lane; j < classes; j += 32) s += expf(x[j] - m);
+    s = warp_sum(s);
+    const float ls = logf(s);
+    float l = 0.f;
+    for (int j = lane; j < classes; j += 32) {
+        const float d = x[j] - m;
+        const float gj = g[j];
+        const float lp = (d < -745.13f) ? -INFINITY : d - ls;
+        l += gj * lp;
+        if (grad) grad[r * classes + j] = (expf(d) / s - gj) * inv;
+    }
+    l = warp_sum(l);
+    if (lane == 0) row_loss[r] = l;
+}
+
 __global__ void __launch_bounds__(kThreads) softmax_ce_kernel(const float* __restrict__ logits,
                                                               const float* __restrict__ gt,
                                                               float* __restrict__ grad,
@@ -158,31 +290,48 @@ __global__ void __launch_bounds__(kThreads) softmax_ce_kernel(const float* __res
     const int lane = threadIdx.x & 31;
     const int64_t warps = (int64_t)gridDim.x * (kThreads / 32);
     const float inv_b = 1.f / (float)batch;
+    for (int64_t r = (int64_t)blockIdx.x * (kThreads / 32) + (threadIdx.x >> 5); r < batch; r += warps)
+        softmax_ce_row(logits, gt, grad, row_loss, r, classes, inv_b, lane);
+}
+
+// Is row r inside one of the [first, end) ranges?  Binary search for the last range with first <= r: the ranges are
+// sorted by `first` (ragged_analysis gives them so); any other table makes the answer wrong, never an access out of
+// bounds, since r itself is always a row of the batch.
+__device__ __forceinline__ bool row_in_ranges(const int32_t* __restrict__ ranges, int64_t n_ranges, int64_t r) {
+    int64_t lo = 0, hi = n_ranges;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if ((int64_t)__ldg(ranges + 2 * mid) <= r) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo > 0 && r < (int64_t)__ldg(ranges + 2 * (lo - 1) + 1);
+}
+
+// softmax_ce_kernel over the rows of the ranges; every other row gets row_loss 0 and a zero gradient row
+__global__ void __launch_bounds__(kThreads) softmax_ce_rows_kernel(const float* __restrict__ logits,
+                                                                   const float* __restrict__ gt,
+                                                                   float* __restrict__ grad,
+                                                                   float* __restrict__ row_loss,
+                                                                   const int32_t* __restrict__ ranges,
+                                                                   int64_t n_ranges, int64_t batch, int classes,
+                                                                   float denom) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warps = (int64_t)gridDim.x * (kThreads / 32);
+    const float inv = 1.f / denom;
     for (int64_t r = (int64_t)blockIdx.x * (kThreads / 32) + (threadIdx.x >> 5); r < batch; r += warps) {
-        const float* x = logits + r * classes;
-        const float* g = gt + r * classes;
-        float m = -INFINITY;
-        for (int j = lane; j < classes; j += 32) m = fmaxf(m, x[j]);
-        m = warp_max(m);
-        float s = 0.f;
-        for (int j = lane; j < classes; j += 32) s += expf(x[j] - m);
-        s = warp_sum(s);
-        const float ls = logf(s);
-        float l = 0.f;
-        for (int j = lane; j < classes; j += 32) {
-            const float d = x[j] - m;
-            const float gj = g[j];
-            const float lp = (d < -745.13f) ? -INFINITY : d - ls;
-            l += gj * lp;
-            if (grad) grad[r * classes + j] = (expf(d) / s - gj) * inv_b;
+        if (row_in_ranges(ranges, n_ranges, r)) {
+            softmax_ce_row(logits, gt, grad, row_loss, r, classes, inv, lane);
+            continue;
         }
-        l = warp_sum(l);
-        if (lane == 0) row_loss[r] = l;
+        if (grad)
+            for (int j = lane; j < classes; j += 32) grad[r * classes + j] = 0.f;
+        if (lane == 0) row_loss[r] = 0.f;
     }
 }
 
-__global__ void __launch_bounds__(1024) neg_mean_kernel(const float* __restrict__ v, int64_t n,
-                                                        float* __restrict__ out) {
+// out = -sum(v[0:n]) / denom, in double
+__device__ __forceinline__ void neg_sum_over(const float* __restrict__ v, int64_t n, double denom,
+                                             float* __restrict__ out) {
     __shared__ double part[32];
     double acc = 0.0;
     for (int64_t i = threadIdx.x; i < n; i += 1024) acc += (double)v[i];
@@ -191,8 +340,18 @@ __global__ void __launch_bounds__(1024) neg_mean_kernel(const float* __restrict_
     __syncthreads();
     if (threadIdx.x < 32) {
         double r = warp_sum(part[threadIdx.x]);
-        if (threadIdx.x == 0) out[0] = (float)(-r / (double)n);
+        if (threadIdx.x == 0) out[0] = (float)(-r / denom);
     }
+}
+
+__global__ void __launch_bounds__(1024) neg_mean_kernel(const float* __restrict__ v, int64_t n,
+                                                        float* __restrict__ out) {
+    neg_sum_over(v, n, (double)n, out);
+}
+
+__global__ void __launch_bounds__(1024) neg_sum_over_kernel(const float* __restrict__ v, int64_t n, float denom,
+                                                            float* __restrict__ out) {
+    neg_sum_over(v, n, (double)denom, out);
 }
 
 // ---------------------------------------------------------------- sigmoid cross-entropy
@@ -361,6 +520,62 @@ int uocr_seg_grad(const float* gt, const float* x_pre, float* out, int64_t n, in
     if (x_pre) seg_grad_kernel<true><<<grid, kThreads, 0, st>>>(gt, coef, x_pre, out, hw, (int)c);
     else seg_grad_kernel<false><<<grid, kThreads, 0, st>>>(gt, coef, nullptr, out, hw, (int)c);
     UOCR_LAUNCHED("seg_grad");
+    return UOCR_OK;
+}
+
+int uocr_seg_loss_ragged(int kind, const float* pred, const float* gt, float* grad, float* loss,
+                         const int32_t* extents, int64_t n, int64_t h, int64_t w, int64_t c, void* workspace,
+                         void* stream) {
+    UOCR_REQUIRE(kind == UOCR_SEG_DICE || kind == UOCR_SEG_JACCARD, "unknown segmentation loss %d", kind);
+    UOCR_REQUIRE(pred && gt && loss && extents && workspace, "NULL pointer");
+    UOCR_REQUIRE(n > 0 && h > 0 && w > 0 && c > 0 && n < 65536 && c < 65536, "bad dimension");
+    cudaStream_t st = as_stream(stream);
+    const int64_t nc = n * c;
+    double* sums = reinterpret_cast<double*>(workspace);
+    float* coef = reinterpret_cast<float*>(sums + 3 * nc);
+    UOCR_CUDA(cudaMemsetAsync(sums, 0, 3 * nc * sizeof(double), st));
+    int64_t chunks = ceil_div(h * w * c, (int64_t)kThreads * 16);
+    const int64_t cap = ceil_div(148 * 8, n);
+    if (chunks > cap) chunks = cap;
+    if (chunks > h) chunks = h;
+    if (chunks < 1) chunks = 1;
+    seg_sums_ragged_kernel<<<dim3((unsigned)chunks, (unsigned)n), kThreads, 0, st>>>(pred, gt, extents, sums, h, w,
+                                                                                     (int)c, nc);
+    UOCR_LAUNCHED("seg_sums_ragged");
+    seg_finalize_kernel<<<1, kThreads, 0, st>>>(kind, sums, coef, nc, loss);
+    UOCR_LAUNCHED("seg_finalize");
+    if (grad) return uocr_seg_grad_ragged(gt, nullptr, grad, extents, n, h, w, c, workspace, stream);
+    return UOCR_OK;
+}
+
+int uocr_seg_grad_ragged(const float* gt, const float* x_pre, float* out, const int32_t* extents, int64_t n,
+                         int64_t h, int64_t w, int64_t c, const void* workspace, void* stream) {
+    UOCR_REQUIRE(gt && out && extents && workspace, "NULL pointer");
+    UOCR_REQUIRE(n > 0 && h > 0 && w > 0 && c > 0 && n < 65536 && c < 65536, "bad dimension");
+    cudaStream_t st = as_stream(stream);
+    const float* coef = reinterpret_cast<const float*>(reinterpret_cast<const double*>(workspace) + 3 * n * c);
+    int64_t blocks = ceil_div(n * h, kThreads / 32);
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    if (x_pre) seg_grad_ragged_kernel<true><<<(int)blocks, kThreads, 0, st>>>(gt, coef, x_pre, out, extents, n, h, w, (int)c);
+    else seg_grad_ragged_kernel<false><<<(int)blocks, kThreads, 0, st>>>(gt, coef, nullptr, out, extents, n, h, w, (int)c);
+    UOCR_LAUNCHED("seg_grad_ragged");
+    return UOCR_OK;
+}
+
+int uocr_softmax_ce_rows(const float* logits, const float* gt, float* grad, float* loss, const int32_t* ranges,
+                         int64_t n_images, int64_t batch, int64_t classes, float denom, float* workspace,
+                         void* stream) {
+    UOCR_REQUIRE(logits && gt && loss && ranges && workspace, "NULL pointer");
+    UOCR_REQUIRE(n_images > 0 && batch > 0 && classes > 0 && classes < (1 << 30), "bad dimension");
+    UOCR_REQUIRE(denom > 0.f, "denominator %g must be positive", (double)denom);
+    cudaStream_t st = as_stream(stream);
+    int64_t blocks = ceil_div(batch, kThreads / 32);
+    if (blocks > 148 * 8) blocks = 148 * 8;
+    softmax_ce_rows_kernel<<<(int)blocks, kThreads, 0, st>>>(logits, gt, grad, workspace, ranges, n_images, batch,
+                                                             (int)classes, denom);
+    UOCR_LAUNCHED("softmax_ce_rows");
+    neg_sum_over_kernel<<<1, 1024, 0, st>>>(workspace, batch, denom, loss);
+    UOCR_LAUNCHED("softmax_ce_rows_loss");
     return UOCR_OK;
 }
 

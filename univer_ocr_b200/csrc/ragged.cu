@@ -8,12 +8,6 @@
 namespace uocr {
 namespace {
 
-__device__ __forceinline__ void ragged_extent(const int32_t* __restrict__ ext, int64_t i, int64_t h, int64_t w,
-                                              int64_t& hi, int64_t& wi) {
-    hi = min((int64_t)max(__ldg(ext + 2 * i), 0), h);
-    wi = min((int64_t)max(__ldg(ext + 2 * i + 1), 0), w);
-}
-
 // One warp per canvas row (image, y).  A row inside the extent zeroes its columns [w_i, W); a row below it is zeroed
 // whole.  Rows wholly inside cost the extent lookup only, so the kernel's traffic is the padding, not the tensor.
 __global__ void __launch_bounds__(kThreads) zero_outside_kernel(float* __restrict__ x, const int32_t* __restrict__ ext,

@@ -26,10 +26,13 @@ class LazySegGrad:
         n, h, w, c = self.shape
         return n, h * w, c
 
+    def _grad(self, x_pre_ptr, out_ptr):
+        lib.uocr_seg_grad(self._gt.ptr, x_pre_ptr, out_ptr, *self._dims(), self._ws.ptr, stream())
+
     def materialize(self):
         if self._dense is None:
             out = DeviceArray(self.shape)
-            lib.uocr_seg_grad(self._gt.ptr, None, out.ptr, *self._dims(), self._ws.ptr, stream())
+            self._grad(None, out.ptr)
             self._dense = out
         return self._dense
 
@@ -38,7 +41,7 @@ class LazySegGrad:
         if self._dense is not None:
             return None
         dx = DeviceArray(self.shape)
-        lib.uocr_seg_grad(self._gt.ptr, x_pre.ptr, dx.ptr, *self._dims(), self._ws.ptr, stream())
+        self._grad(x_pre.ptr, dx.ptr)
         return dx
 
     def __radd__(self, other):                              # Model.backward sums fan-out gradients: 0 + g
@@ -58,8 +61,36 @@ class LazySegGrad:
         return self.materialize().__array__(dtype)
 
 
+class LazySegGradRagged(LazySegGrad):
+    """`LazySegGrad` of a ragged batch (`_Segmentation.ragged`): the gradient is written by uocr_seg_grad_ragged, so it
+    is 0 outside each image's extent, with or without the Sigmoid derivative."""
+
+    def __init__(self, gt, workspace, shape, extents, offset):
+        super().__init__(gt, workspace, shape)
+        self._ext, self._off = extents, offset
+
+    def _grad(self, x_pre_ptr, out_ptr):
+        lib.uocr_seg_grad_ragged(self._gt.ptr, x_pre_ptr, out_ptr, self._ext.ptr + 4 * self._off, *self.shape,
+                                 self._ws.ptr, stream())
+
+
 class _Segmentation(BaseLoss):
     kind = None
+
+    def ragged(self, prediction, ground_truth, extents, offset=0, want_grad=True):
+        """The loss of a ragged batch: (N, H, W, C) canvases, image n in its (h_n, w_n) region, the int32 (N, 2) table
+        of those extents at `extents` (a device array) + `offset` int32 elements.  Sums over each region only; the
+        loss is the sum of the per-image losses, as for a stacked batch."""
+        pred, gt = as_device(prediction), as_device(ground_truth)
+        assert pred.shape == gt.shape and pred.ndim == 4, f'{pred.shape} vs {gt.shape}'
+        n, h, w, c = pred.shape
+        need = ctypes.c_size_t(0)
+        lib.uocr_seg_loss_workspace(n, c, ctypes.byref(need))
+        ws = DeviceArray((need.value + 7) // 8, 'float64')
+        loss = DeviceArray((1,))
+        lib.uocr_seg_loss_ragged(self.kind, pred.ptr, gt.ptr, None, loss.ptr, extents.ptr + 4 * offset, n, h, w, c,
+                                 ws.ptr, stream())
+        return LazyScalar(loss), (LazySegGradRagged(gt, ws, pred.shape, extents, offset) if want_grad else None)
 
     def __call__(self, prediction, ground_truth, want_grad=True):
         pred, gt = as_device(prediction), as_device(ground_truth)
@@ -109,4 +140,18 @@ class SoftmaxCrossEntropy(BaseLoss):
         grad = DeviceArray(pred.shape) if want_grad else None
         lib.uocr_softmax_ce(pred.ptr, gt.ptr, grad.ptr if want_grad else None, loss.ptr, batch,
                             classes, ws.ptr, stream())
+        return LazyScalar(loss), grad
+
+    def rows(self, prediction, ground_truth, ranges, offset, n_ranges, denom, want_grad=True):
+        """The loss over the rows of a windowed ragged batch: the int32 (n_ranges, 2) [first, end) table at `ranges` (a
+        device array) + `offset` int32 elements.  loss = -sum(gt * log p) over those rows / denom; every other row adds
+        nothing and gets a zero gradient."""
+        pred, gt = as_device(prediction), as_device(ground_truth)
+        assert pred.shape == gt.shape and pred.ndim == 2, f'{pred.shape} vs {gt.shape}'
+        batch, classes = pred.shape
+        loss = DeviceArray((1,))
+        ws = DeviceArray((batch,))
+        grad = DeviceArray(pred.shape) if want_grad else None
+        lib.uocr_softmax_ce_rows(pred.ptr, gt.ptr, grad.ptr if want_grad else None, loss.ptr,
+                                 ranges.ptr + 4 * offset, n_ranges, batch, classes, float(denom), ws.ptr, stream())
         return LazyScalar(loss), grad

@@ -16,6 +16,7 @@ memoised recursion per call, the evaluation order is resolved once at `initializ
 replayed; no layer call synchronises the device, and loss values stay on the device until read.
 """
 import ctypes
+from collections import namedtuple
 
 import numpy as np
 
@@ -24,7 +25,7 @@ from .gpu import CP, DeviceArray, LazyScalar, as_device, stream
 from .help_func import make_list_if_not
 from .layers import (BaseLayer, Conv2DToBatchedFixedWidthed, Convolutional2D, Flatten, FromOutput, FullyConnected,
                      LeakyRelu, Relu, Sigmoid, Upsample2D, _kmajor_copy)
-from .losses import SoftmaxCrossEntropy
+from .losses import SegmentationDice2D, SegmentationJaccard2D, SoftmaxCrossEntropy
 from .progress_tracker import track_method
 
 
@@ -462,10 +463,12 @@ class Model(BaseModel):
         outputs[a2_name if a2_name is not None else c2_name] = y
 
     @track_method('backward')
-    def backward(self, grads, on_layer_done=None):
+    def backward(self, grads, on_layer_done=None, plan=None, after_layer=None):
         """`on_layer_done(name)` is called as soon as the parameter gradients of layer `name` are final (its backward
         kernels are queued on the current stream) -- the data-parallel step starts that layer's gradient allreduce
-        there, while the rest of backward runs."""
+        there, while the rest of backward runs.  `plan`: the step plan the forward ran (default: the training plan),
+        whose fused pairs run their fused backward.  `after_layer(name, input_grads)` is called after each layer's
+        backward (the ragged step masks the input gradients there)."""
         grads = make_list_if_not(grads)
         produced = {}                                               # layer -> list of input grads
         done = on_layer_done if on_layer_done is not None else (lambda name: None)
@@ -477,7 +480,7 @@ class Model(BaseModel):
             return sum(parts)                                       # 0 + g1 (+ g2 ...), reference :218
 
         pairs = {}                                                  # member layer -> ('pair', c1, a1, c2, None)
-        for step in self._plan_train:
+        for step in (plan if plan is not None else self._plan_train):
             if step[0] == 'pair':
                 for member in step[1:4]:
                     pairs[member] = step
@@ -492,6 +495,8 @@ class Model(BaseModel):
                     produced[name] = [None] * len(self.relations[name])
                 else:
                     produced[name] = make_list_if_not(layer.backward(incoming(name)))
+                if after_layer is not None:
+                    after_layer(name, produced[name])
                 done(name)
             elif name == step[3]:                                   # conv_2: keep its output gradient
                 stash[step[1]] = incoming(name)
@@ -502,6 +507,8 @@ class Model(BaseModel):
                 first = all(isinstance(src, int) for src in self.relations[name])
                 produced[name] = [self._pair_backward(step, stash.pop(name),
                                                       need_dx=self.compute_input_grads or not first)]
+                if after_layer is not None:
+                    after_layer(name, produced[name])
                 done(step[3])
                 done(name)
         for key in range(self.inputs_count):
@@ -572,23 +579,32 @@ class Model(BaseModel):
     def train_fused(self, X, y, reduce_gradients=None, grad_scale=1.0, on_layer_done=None):
         """One training step on the flat buffers.  `reduce_gradients()` runs between backward and the update (the
         data-parallel allreduce); returns the same dict as `train`."""
-        opt, flat = self.fused_optimizer(), self.flat_parameters()
-        assert flat is not None and opt is not None, 'model does not qualify for the fused update'
-        if not flat.attached():
-            flat.adopt()
-        if not flat.clean:
-            flat.zero_grads()
         X, y = make_list_if_not(X), make_list_if_not(y)
-        keep, self.compute_input_grads = self.compute_input_grads, False    # `train` never surfaces dL/dX (:250-254)
-        try:
+
+        def step():
             predicted = self.forward(X, clear_grads=False)
             losses, gradients = [], []
             for key in range(self.outputs_count):
                 loss, grad = self._loss_for(key)(predicted[key], y[key])
                 losses.append(loss)
                 gradients.append(grad)
-            flat.clean = False
+            self._flat.clean = False
             self.backward(gradients, on_layer_done=on_layer_done)
+            return losses
+        return self._fused_step(step, reduce_gradients, grad_scale)
+
+    def _fused_step(self, step, reduce_gradients, grad_scale):
+        """`step()` (forward + loss + backward into the flat gradient buffer -> output losses) between the flat
+        buffers' set-up and the fused update."""
+        opt, flat = self.fused_optimizer(), self.flat_parameters()
+        assert flat is not None and opt is not None, 'model does not qualify for the fused update'
+        if not flat.attached():
+            flat.adopt()
+        if not flat.clean:
+            flat.zero_grads()
+        keep, self.compute_input_grads = self.compute_input_grads, False    # `train` never surfaces dL/dX (:250-254)
+        try:
+            losses = step()
         finally:
             self.compute_input_grads = keep
         if reduce_gradients is not None:
@@ -710,32 +726,189 @@ class Model(BaseModel):
         def out_table(src):
             return ext.copy() if isinstance(src, int) else modes[src][1].copy()
 
-        # every extent table a kernel reads, uploaded in one copy: the input's, then one per masked output
-        tables, offsets = [ext], {}
-        for name in self._order:
-            kind, table, canvas_hw = modes[name]
-            if kind == 'hw' and ((table[:, 0] < canvas_hw[0]) | (table[:, 1] < canvas_hw[1])).any():
-                offsets[name] = sum(t.size for t in tables)
-                tables.append(table)
-        dev = DeviceArray.from_host(np.concatenate(tables).astype(np.int32), np.int32)
-        X = as_device(canvas)
+        dev, masked, _ = self._ragged_tables(ext, modes, canvas.shape[1:3])
+        outputs = self._infer_ragged(as_device(canvas), ext, dev, masked)
+        return outputs, [out_table(src) for src in out_names]
+
+    def _infer_ragged(self, X, ext, dev, masked):
         if self._fusion_planned and isinstance(self.infer_fusion, HourglassFusion):
             fused = self.infer_fusion(self, [X], ext, dev.ptr)
             if fused is not None:
                 self.layers_outputs = {**{name: None for name in self.layers}, 0: fused[0]}
-                return fused, [out_table(out_names[0])]
+                return fused
         if self._plan_ragged is None:
             self._plan_ragged = self._make_plan(training=False, ragged=True) if self._fusion_planned else self._plan_infer
+        outputs = self._run_steps(self._plan_ragged, [X], False, True, after_step=self._ragged_mask(dev, masked))
+        self.layers_outputs = outputs
+        return [outputs[k] for k in range(self.outputs_count)]
 
+    def _ragged_tables(self, ext, modes, canvas_hw, loss_keys=()):
+        """Every int32 table the kernels of a ragged batch read, uploaded in one copy: the input's extents first (the Line
+        one-kernel reads them there), then the table of every image map with an extent smaller than its canvas -- the
+        maps that are masked -- and, for the outputs in `loss_keys`, the table their loss reads.  -> (device tables,
+        {source (layer name, or 0 for the input): offset of its table}, {output index: offset of its loss table}).  An
+        output without an entry has no padding: its loss is the stacked batch's."""
+        def padded(table, hw):
+            return bool(((table[:, 0] < hw[0]) | (table[:, 1] < hw[1])).any())
+
+        tables, masked, at = [ext], {}, {}
+        if padded(ext, canvas_hw):
+            masked[0] = 0
+        for name in self._order:
+            kind, table, hw = modes[name]
+            if kind == 'hw' and padded(table, hw):
+                masked[name] = sum(t.size for t in tables)
+                tables.append(table)
+        for key in loss_keys:
+            src = self.relations[key][0]
+            if src in masked:
+                at[key] = masked[src]
+            elif not isinstance(src, int) and modes[src][0] == 'rows':
+                at[key] = sum(t.size for t in tables)
+                tables.append(modes[src][1])
+        return DeviceArray.from_host(np.concatenate(tables).astype(np.int32), np.int32), masked, at
+
+    @staticmethod
+    def _ragged_mask(dev, masked):
+        """after_step of a ragged forward: zero the step's output outside each extent where some extent is smaller
+        than the canvas."""
         def mask(step, outputs):
             name = [m for m in step[1:] if m is not None][-1]
-            if name in offsets:
+            if name in masked:
                 y = outputs[name]
-                lib.uocr_zero_outside_hw_f32(y.ptr, dev.ptr + 4 * offsets[name], *y.shape, stream())
+                lib.uocr_zero_outside_hw_f32(y.ptr, dev.ptr + 4 * masked[name], *y.shape, stream())
+        return mask
 
-        outputs = self._run_steps(self._plan_ragged, [X], False, True, after_step=mask)
+    # ---- ragged training ------------------------------------------------------------
+    # A parameter gradient over the canvas (sum x * dy, sum dy) is the sum of the per-image gradients when every saved
+    # forward map and every gradient map is zero outside its image's extent (DESIGN.md §3).  The forward masks see to
+    # the first; for the second, the loss gradient is 0 outside the extents (or row ranges), and after the backward of
+    # each layer that spreads a gradient into the padding -- a convolution's dgrad, the window layer's scatter -- its
+    # input gradients are zeroed outside their extents.  Elementwise layers map a zero gradient to zero and
+    # Upsample2D's block sum keeps the zeros, so they need no mask.
+    RAGGED_LOSSES = (SegmentationDice2D, SegmentationJaccard2D, SoftmaxCrossEntropy)
+    RAGGED_SPREADING = (Convolutional2D, Conv2DToBatchedFixedWidthed)
+    _plan_train_ragged = None
+    _RaggedBatch = namedtuple('_RaggedBatch', 'ext modes targets dev masked loss_at plan')
+
+    def ragged_train_analysis(self, canvas_shape, extents, y):
+        """`ragged_analysis` of a training batch, plus the checks of its targets `y` (one per output), all on the host:
+        a Dice / Jaccard output is an image map and its target is that output's (N, H', W', C') canvas, image i in its
+        region; a SoftmaxCrossEntropy output comes after a Conv2DToBatchedFixedWidthed and its target has the
+        (N * W', classes) rows of that output, image i's labels in rows [i * W', i * W' + w_i).  Raises ValueError for
+        any other loss, for targets of another shape and for everything ragged_analysis rejects.  -> (extents, modes)
+        as ragged_analysis."""
+        for key in range(self.outputs_count):
+            if type(self._loss_for(key)) not in self.RAGGED_LOSSES:
+                raise ValueError(f'output {key}: {type(self._loss_for(key)).__name__} is not supported on ragged batches')
+        ext, modes = self.ragged_analysis(canvas_shape, extents)
+        ys = make_list_if_not(y)
+        if len(ys) != self.outputs_count:
+            raise ValueError(f'{len(ys)} targets for {self.outputs_count} outputs')
+        out_shapes = self.get_output_shapes([tuple(int(v) for v in canvas_shape)])
+        for key, (target, want) in enumerate(zip(ys, out_shapes)):
+            src = self.relations[key][0]
+            rows = not isinstance(src, int) and modes[src][0] == 'rows'
+            loss = self._loss_for(key)
+            if rows != isinstance(loss, SoftmaxCrossEntropy):
+                raise ValueError(f'output {key}: {type(loss).__name__} of '
+                                 f'{"window rows" if rows else "an image map"} is not supported on ragged batches')
+            shape = tuple(int(v) for v in np.shape(target)) if not hasattr(target, 'shape') else tuple(target.shape)
+            if shape != tuple(want):
+                raise ValueError(f'output {key}: target of shape {shape}, the output canvas is {tuple(want)}')
+        return ext, modes
+
+    def _ragged_batch(self, canvas, extents, y, training):
+        """Host checks (nothing is launched before they pass), then the one upload of the tables."""
+        ext, modes = self.ragged_train_analysis(canvas.shape, extents, y)
+        dev, masked, loss_at = self._ragged_tables(ext, modes, canvas.shape[1:3], range(self.outputs_count))
+        plan = None
+        if training:
+            plan = self._plan_train
+            if masked:                      # the Monochrome pair keeps its hidden map on chip: it steps aside
+                if self._plan_train_ragged is None:
+                    self._plan_train_ragged = (self._make_plan(training=True, ragged=True) if self._fusion_planned
+                                               else self._plan_train)
+                plan = self._plan_train_ragged
+        return self._RaggedBatch(ext, modes, make_list_if_not(y), dev, masked, loss_at, plan)
+
+    def _ragged_losses(self, predicted, batch, rows_total, want_grad):
+        losses, gradients = [], []
+        for key in range(self.outputs_count):
+            fn, pred, target = self._loss_for(key), predicted[key], batch.targets[key]
+            if isinstance(fn, SoftmaxCrossEntropy):
+                table = batch.modes[self.relations[key][0]][1]
+                valid = int((table[:, 1] - table[:, 0]).sum())
+                if rows_total is None and valid == pred.shape[0]:         # every row valid: the stacked batch's loss
+                    loss, grad = fn(pred, target, want_grad=want_grad)
+                else:
+                    loss, grad = fn.rows(pred, target, batch.dev, batch.loss_at[key], len(table),
+                                         valid if rows_total is None else rows_total, want_grad=want_grad)
+            elif key in batch.loss_at:
+                loss, grad = fn.ragged(pred, target, batch.dev, batch.loss_at[key], want_grad=want_grad)
+            else:
+                loss, grad = fn(pred, target, want_grad=want_grad)
+            losses.append(loss)
+            gradients.append(grad)
+        return losses, gradients
+
+    def _ragged_pass(self, X, batch, rows_total, clear_grads, on_layer_done=None):
+        """Forward (masked), loss over the extents / row ranges and backward (input gradients masked) -> output losses."""
+        outputs = self._run_steps(batch.plan, [X], True, clear_grads, after_step=self._ragged_mask(batch.dev, batch.masked))
         self.layers_outputs = outputs
-        return [outputs[k] for k in range(self.outputs_count)], [out_table(src) for src in out_names]
+        losses, gradients = self._ragged_losses([outputs[k] for k in range(self.outputs_count)], batch, rows_total, True)
+        dev, masked = batch.dev, batch.masked
+
+        def mask_input_grads(name, grads):
+            if type(self.layers[name]) not in self.RAGGED_SPREADING:
+                return
+            for src, g in zip(self.relations[name], grads):
+                if g is not None and src in masked:
+                    lib.uocr_zero_outside_hw_f32(g.ptr, dev.ptr + 4 * masked[src], *g.shape, stream())
+
+        self.backward(gradients, on_layer_done=on_layer_done, plan=batch.plan,
+                      after_layer=mask_input_grads if masked else None)
+        return losses
+
+    def compute_loss_and_gradients_ragged(self, canvas, extents, y, rows_total=None):
+        """`compute_loss_and_gradients` of a ragged batch: `canvas` (N, H, W, C), zero outside each image, image i in
+        canvas[i, :h_i, :w_i, :]; `extents` host (N, 2) integers (h_i, w_i); `y` the targets on the output canvases
+        (see ragged_train_analysis).  Dice / Jaccard losses are the sum of the per-image losses; SoftmaxCrossEntropy is
+        the mean over the valid rows, or their sum over `rows_total` when given (a data-parallel step passes the valid
+        rows of all ranks).  With no padding both equal the stacked batch's loss.  The parameter gradients are those of
+        the loss, i.e. the per-image gradients summed (Dice) or weighted by w_i / sum(w) (SoftmaxCE)."""
+        batch = self._ragged_batch(canvas, extents, y, training=True)
+        if self._flat:
+            self._flat.clean = False                                # gradients are about to be left in param.grad
+        losses = self._ragged_pass(as_device(canvas), batch, rows_total, clear_grads=True)
+        return {'output_losses': losses, 'regularization_loss': self.regularize()}
+
+    def train_fused_ragged(self, canvas, extents, y, rows_total=None, reduce_gradients=None, grad_scale=1.0,
+                           on_layer_done=None):
+        """`train_fused` of a ragged batch (arguments as compute_loss_and_gradients_ragged)."""
+        batch = self._ragged_batch(canvas, extents, y, training=True)
+        X = as_device(canvas)
+
+        def step():
+            self._flat.clean = False
+            return self._ragged_pass(X, batch, rows_total, clear_grads=False, on_layer_done=on_layer_done)
+        return self._fused_step(step, reduce_gradients, grad_scale)
+
+    def train_ragged(self, canvas, extents, y, rows_total=None):
+        """`train` of a ragged batch: the fused flat update when the model qualifies, else the per-parameter route."""
+        if self.fused_update and self.fused_optimizer() is not None:
+            return self.train_fused_ragged(canvas, extents, y, rows_total=rows_total)
+        losses = self.compute_loss_and_gradients_ragged(canvas, extents, y, rows_total=rows_total)
+        self.update_grads()
+        self.clear_grads()
+        return losses
+
+    def test_ragged(self, canvas, extents, y):
+        """`test` of a ragged batch: the inference path of predict_ragged, then the losses of the training step."""
+        batch = self._ragged_batch(canvas, extents, y, training=False)
+        predicted = self._infer_ragged(as_device(canvas), batch.ext, batch.dev, batch.masked)
+        losses, _ = self._ragged_losses(predicted, batch, None, want_grad=False)
+        return {'output_losses': losses}
 
     def update_grads(self):
         if not self.trainable:

@@ -17,7 +17,8 @@ can be replayed from one CUDA graph (`pipeline.CapturedStep`).
 
 Gradient scaling: the Dice / Jaccard losses sum over the batch (`losses.py:23`), so shard gradients are summed
 without scaling; SoftmaxCE / SigmoidCE divide by the LOCAL batch (`losses.py:69-72`), so their summed gradients are
-scaled by 1 / world (= local / global batch).  The L2 gradient depends on the weights only, so it is added once,
+scaled by 1 / world (= local / global batch).  A ragged SoftmaxCE step (`train_ragged` with `rows_total`) divides by
+the valid rows of all ranks instead and is not scaled.  The L2 gradient depends on the weights only, so it is added once,
 after the allreduce (inside the fused update).
 """
 import ctypes
@@ -125,6 +126,23 @@ class DataParallel:
         hook = self._layer_done if self.overlap else None
         out = self.model.train_fused(X, y, reduce_gradients=self._reduce, grad_scale=self.grad_scale,
                                      on_layer_done=hook)
+        return self._finish(out)
+
+    def train_ragged(self, canvas, extents, y, rows_total=None):
+        """`train` on this rank's ragged batch (Model.train_fused_ragged).  Dice / Jaccard losses sum over images, so
+        the summed gradients are the global ones.  A mean-over-rows loss given `rows_total`, the valid rows of all
+        ranks, is already divided by the global count, so its summed gradients are not scaled either; without it the
+        1 / world rule of `train` applies."""
+        self.scheduler.reset()
+        self.buckets_last_step = []
+        hook = self._layer_done if self.overlap else None
+        scale = 1.0 if rows_total is not None else self.grad_scale
+        out = self.model.train_fused_ragged(canvas, extents, y, rows_total=rows_total, reduce_gradients=self._reduce,
+                                            grad_scale=scale, on_layer_done=hook)
+        return self._finish(out)
+
+    @staticmethod
+    def _finish(out):
         if not isinstance(out['regularization_loss'], LazyScalar):
             out['regularization_loss'] = LazyScalar(_zero_scalar())
         return out

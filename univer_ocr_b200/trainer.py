@@ -30,6 +30,15 @@ Losses that average over the local batch (SoftmaxCE / SigmoidCE, `nn/losses.py:6
 weighted by the number of stacked samples so that an epoch's sum equals the reference's sum of
 per-sample losses (exactly for equal sample sizes); Dice / Jaccard already sum over the batch.
 
+Samples of different sizes -- the reference's data: pages, paragraph crops and line crops differ in
+size -- are batched too.  When a model's samples in a batch differ in any axis but the first, they
+are packed on the host instead of stacked: X on a zero-filled (N, H, W, C) canvas with each image's
+(h, w) in a table of extents, y on its output canvas (image maps) or in its row ranges (window
+rows), and the batch runs through `train_ragged` / `test_ragged` (`Model.train_ragged`, DESIGN.md
+§3).  At world > 1 a mean-over-batch model's training step sums [ragged?, valid rows, samples] over
+the ranks with one `allreduce_host`, so that every rank takes the same path; a ragged step then
+divides its loss by the valid rows of all ranks and is weighted by the samples of all ranks.
+
 Any object with `train(X, y) / test(X, y) / get_weights() / set_weights(w) / nan_weights() /
 get_outputs_count()` is accepted as a model (used as is); `nn.models.Model` instances are wrapped
 in `DataParallel` unless `fused_update=False`.
@@ -174,6 +183,12 @@ class _Stepper:
     def test(self, X, y):
         return self.model.test(X, y)
 
+    def train_ragged(self, canvas, extents, y, rows_total=None):
+        return (self.dp or self.model).train_ragged(canvas, extents, y, rows_total=rows_total)
+
+    def test_ragged(self, canvas, extents, y):
+        return self.model.test_ragged(canvas, extents, y)
+
     def snapshot(self):
         if self.dp is None:
             return self.model.get_weights()
@@ -251,6 +266,59 @@ class Trainer:
             return items[0] if len(items) == 1 else np.concatenate(items, axis=0)
         return cat([p[0] for p in parts]), cat([p[1] for p in parts])
 
+    @staticmethod
+    def _ragged(parts):
+        """True when the parts' X are image batches that differ in an axis other than the first (cannot be stacked)."""
+        xs = [p[0] for p in parts]
+        if any(isinstance(x, (list, tuple)) or np.ndim(x) != 4 for x in xs):
+            return False
+        return len({tuple(np.shape(x)[1:]) for x in xs}) > 1
+
+    @staticmethod
+    def _pack(parts):
+        """[(X, y), ...] with X (k, h, w, C) of different sizes -> (canvas, extents, y, valid rows): X on a zero-filled
+        (N, H, W, C) canvas, (H, W) the largest extents, a part with k images adding k rows (h, w) to the table.  A
+        target that is an image map, (k, h', w', C'), goes on its zero-filled canvas the same way; one of window rows,
+        (k * r, classes), puts image j's r rows at [j * R, j * R + r), R the largest r -- the layout of
+        Model.ragged_train_analysis, since a network's output extents grow with its input's.  Valid rows: the rows of
+        the first target (0 for image maps)."""
+        xs = [np.asarray(p[0]) for p in parts]
+        counts = [x.shape[0] for x in xs]
+        n = sum(counts)
+        canvas = np.zeros((n, max(x.shape[1] for x in xs), max(x.shape[2] for x in xs), xs[0].shape[3]), np.float32)
+        ext = np.zeros((n, 2), np.int64)
+        i = 0
+        for x in xs:
+            canvas[i:i + x.shape[0], :x.shape[1], :x.shape[2]] = x
+            ext[i:i + x.shape[0]] = x.shape[1:3]
+            i += x.shape[0]
+
+        def place(items):
+            if isinstance(items[0], (list, tuple)):
+                return [place([it[k] for it in items]) for k in range(len(items[0]))]
+            ts = [np.asarray(t) for t in items]
+            if ts[0].ndim == 4:
+                out = np.zeros((n, max(t.shape[1] for t in ts), max(t.shape[2] for t in ts), ts[0].shape[3]), np.float32)
+                j = 0
+                for t in ts:
+                    out[j:j + t.shape[0], :t.shape[1], :t.shape[2]] = t
+                    j += t.shape[0]
+                return out
+            per = [t.shape[0] // k for t, k in zip(ts, counts)]
+            rows = max(per)
+            out = np.zeros((n * rows, *ts[0].shape[1:]), np.float32)
+            j = 0
+            for t, k, r in zip(ts, counts, per):
+                for m in range(k):
+                    out[(j + m) * rows:(j + m) * rows + r] = t[m * r:(m + 1) * r]
+                j += k
+            return out
+
+        y = place([p[1] for p in parts])
+        first = [np.asarray(p[1][0] if isinstance(p[1], (list, tuple)) else p[1]) for p in parts]
+        valid = sum(t.shape[0] for t in first) if first[0].ndim == 2 else 0
+        return canvas, ext, y, valid
+
     def _batches(self, dataset, order):
         """`_host_batches` with the next `prefetch` batches fetched and stacked by a background thread while the
         current one trains (host data sets only: `get_batch` data sets do their own staging)."""
@@ -291,8 +359,9 @@ class Trainer:
             stop.set()
 
     def _host_batches(self, dataset, order):
-        """Yields ({name: (X, y, n_samples)}, samples consumed so far): `batch_size` samples per
-        step, this rank's share [rank::world] of each."""
+        """Yields ({name: (X, y, n_samples, ragged)}, samples consumed so far): `batch_size` samples per
+        step, this rank's share [rank::world] of each.  `ragged` is None for a stacked batch, else (extents, valid
+        rows) of a packed one (X, y its canvases, `_pack`)."""
         batched = getattr(dataset, 'get_batch', None)
         for start in range(0, len(order), self.batch_size):
             chunk = order[start:start + self.batch_size]
@@ -306,7 +375,8 @@ class Trainer:
             if batched is not None:
                 # the data set stacks (and may keep its samples on the device): {name: (X, y)} for these indices
                 got = batched(mine)
-                yield {name: (X, y, len(mine)) for name, (X, y) in got.items() if name in self.models}, start + len(chunk)
+                yield ({name: (X, y, len(mine), None) for name, (X, y) in got.items() if name in self.models},
+                   start + len(chunk))
                 continue
             samples = [dataset.get(i) for i in mine]
             batch = {}
@@ -316,9 +386,12 @@ class Trainer:
                     raise ValueError(f'data-parallel training needs every model in every sample: {name!r} is missing '
                                      f'from {len(samples) - len(parts)} of this rank\'s {len(samples)} samples (a rank '
                                      f'that skips a model\'s step leaves the others waiting in its allreduce)')
-                if parts:
+                if parts and self._ragged(parts):
+                    X, ext, y, valid = self._pack(parts)
+                    batch[name] = (X, y, len(parts), (ext, valid))
+                elif parts:
                     X, y = self._stack(parts)
-                    batch[name] = (X, y, len(parts))
+                    batch[name] = (X, y, len(parts), None)
             yield batch, start + len(chunk)
 
     def _run(self, dataset, order, training, losses):
@@ -328,13 +401,36 @@ class Trainer:
                 self.progress_tracker.reset()
             self._message('training' if training else 'validating')
             update, weights = {}, {}
-            for name, (X, y, n) in batch.items():
+            agree = training and self.world > 1 and not hasattr(dataset, 'get_batch')
+            for name, (X, y, n, ragged) in batch.items():
                 st = self.steppers[name]
-                update[name] = st.train(X, y) if training else st.test(X, y)
                 weights[name] = n if st.mean_loss else 1
+                if agree and st.mean_loss:
+                    update[name], weights[name] = self._train_mean_step(st, X, y, n, ragged)
+                elif ragged is not None:
+                    ext = ragged[0]
+                    update[name] = st.train_ragged(X, ext, y) if training else st.test_ragged(X, ext, y)
+                else:
+                    update[name] = st.train(X, y) if training else st.test(X, y)
             for name in update:                          # one weight per model
                 (losses.train if training else losses.validation)({name: update[name]}, weights[name])
             self._message('train_iteration' if training else 'val_iteration', {'current': done, 'total': total})
+
+    def _train_mean_step(self, st, X, y, n, ragged):
+        """A mean-over-batch model's training step at world > 1 -> (losses, weight).  The ranks sum [ragged?, valid rows,
+        samples]; if any rank's batch is ragged, every rank takes the ragged step (a stacked batch is a canvas without
+        padding) with the loss over the valid rows of all ranks, weighted by the samples of all ranks."""
+        if ragged is not None:
+            rows = ragged[1]
+        else:
+            first = y[0] if isinstance(y, (list, tuple)) else y
+            rows = np.shape(first)[0] if np.ndim(first) == 2 else 0
+        any_ragged, rows_total, samples = self.comm.allreduce_host([float(ragged is not None), float(rows), float(n)],
+                                                                   'sum')
+        if not any_ragged:
+            return st.train(X, y), n
+        ext = ragged[0] if ragged is not None else np.tile(np.shape(X)[1:3], (np.shape(X)[0], 1))
+        return st.train_ragged(X, ext, y, rows_total=int(round(rows_total))), int(round(samples))
 
     def _usable(self, n):
         """Samples of an n-sample data set that a pass consumes (all of them on one rank)."""
